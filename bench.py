@@ -57,7 +57,38 @@ def parse_args():
                          "ordered: point-ordered sums, bit-identical to the reference")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-profile", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the timed path returned in its last step (rank 0) as "
+                         "DIR/<name>.npy in float32, at most 60 MB in all (a fixed, seeded sample of points beyond that), so that "
+                         "two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "lccrf":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl lccrf)")
+    return args
+
+
+DUMP_LIMIT = 60_000_000  # bytes on disk written by --dump-outputs in all, headers included: below 64 MB with room to spare
+NPY_HEADER = 1024        # bytes set aside per .npy file for its header (numpy writes 128 for these arrays)
+
+
+def dump_outputs(out_dir: str, arrays: dict, limit: int = DUMP_LIMIT) -> None:
+    """Writes per-point outputs (first axis = point, the same number of points in every array) as out_dir/<name>.npy
+    in float32.  Outputs whose files would exceed `limit` bytes are sampled: the same fixed, seeded set of points from
+    every array, whose indices go to out_dir/point_index.npy (float32 while that is exact, float64 beyond 2^24 points)."""
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items()}
+    n = next(iter(arrays.values())).shape[0]
+    per_point = sum(a.nbytes for a in arrays.values()) // max(n, 1)
+    if n * per_point + NPY_HEADER * len(arrays) > limit:
+        idx_type = np.dtype(np.float32 if n <= 1 << 24 else np.float64)
+        keep = (limit - NPY_HEADER * (len(arrays) + 1)) // (per_point + idx_type.itemsize)
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+        arrays["point_index"] = idx.astype(idx_type)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 WORKLOADS = {
@@ -497,6 +528,7 @@ def run_gpu_arm_image(args):
         launches = ctx.kernel_launches - l0
         clocks = sampler.stop() if sampler else None
         assert all(np.array_equal(a, b) for a, b in zip(maps, ref_maps))  # deterministic
+        timed_maps = list(maps)  # step() below replaces the entries of `maps`
     t_dev = torch.tensor([ms, max(ms, wall_ms)], dtype=torch.float64, device="cuda")
     if dist is not None:
         dist.all_reduce(t_dev, op=dist.ReduceOp.MAX)
@@ -558,6 +590,8 @@ def run_gpu_arm_image(args):
         "gpu_launches": int(launches), "roofline": roofline, "kernel_shares": shares, "kernel_avg_launch_ms": kernel_ms,
         "lattice_vertices": V, "cpu_baseline": cpu,
     }
+    if args.dump_outputs:  # the pixels of this rank's images, one image after the other
+        dump_outputs(args.dump_outputs, {"map_labels": np.concatenate(timed_maps)})
     print(json.dumps(line), flush=True)
     if dist is not None:
         dist.barrier()
@@ -696,9 +730,11 @@ def run_gpu_arm_replay(args):
         ms = elapsed_all(a)
         clocks = sampler.stop() if sampler else None
         # the last step once more against the final map: the pipelined loop delivered exactly these results
+        timed_out = []
         for st, (m_, p_) in zip(S, last):
             m2, p2 = st["F"].get_outputs()
             assert np.array_equal(m_, m2) and np.array_equal(p_.view(np.int32), p2.view(np.int32))
+            timed_out.append((m2, p2))
     t_dev = torch.tensor([ms, ms_e2e], dtype=torch.float64, device="cuda")
     if dist is not None:
         dist.all_reduce(t_dev, op=dist.ReduceOp.MAX)
@@ -784,6 +820,9 @@ def run_gpu_arm_replay(args):
         "gpu_launches": int(launches), "roofline": roofline, "kernel_shares": shares, "kernel_avg_launch_ms": kernel_ms,
         "parity_vs_oracle": parity, "cpu_baseline": cpu,
     }
+    if args.dump_outputs:  # the sequences of this rank, one after the other
+        dump_outputs(args.dump_outputs, {"map_labels": np.concatenate([m for m, _ in timed_out]),
+                                         "marginals": np.concatenate([p for _, p in timed_out])})
     print(json.dumps(line), flush=True)
     if dist is not None:
         dist.barrier()
@@ -916,6 +955,7 @@ def run_gpu_arm(args):
         barrier()
         ms = ev0.elapsed_time(ev1)
         launches = ctx.kernel_launches - l0
+        timed_out = F.get_outputs() if args.dump_outputs else None  # before the loops below run F again
         # the same device-resident loop in the other splat mode (reported beside the headline, never as `value`)
         ms_alt = 0.0
         if not args.no_profile:
@@ -1114,6 +1154,8 @@ def run_gpu_arm(args):
         "step_hbm_frac": (abytes["total"] / (ms / args.steps * 1e-3) / 1e9) / peak,
         "cpu_baseline": cpu,
     }
+    if timed_out is not None:
+        dump_outputs(args.dump_outputs, {"map_labels": timed_out[0], "marginals": timed_out[1]})
     print(json.dumps(line), flush=True)
     if dist is not None:
         dist.barrier()

@@ -26,10 +26,8 @@ def oracle():
 
 @pytest.fixture(scope="session")
 def ref():
-    from oracle.pyoracle import Ref
-    if not Ref.available():
-        pytest.skip("oracle/_ref/libref.so not built (reference tree absent at build time)")
-    return Ref()
+    from util import Reference
+    return Reference()
 
 
 @pytest.fixture(scope="session")

@@ -1,7 +1,8 @@
 """CPU tests: the oracle (oracle/lccrf_oracle.c) is pinned against
   (1) the reference's one golden vector (examples/res1_cpu.ppm -> tests/golden/golden_im1.npz),
   (2) outputs of the UNMODIFIED reference headers stored in tests/golden/golden_ref.npz,
-  (3) the reference headers compiled in place (oracle/_ref/libref.so), when present.
+  (3) the reference headers compiled in place (oracle/_ref/libref.so) on seeded sweeps -- live where that library was
+      built, otherwise against the sweeps' reference outputs stored in tests/golden/golden_ref_sweep.npz.
 """
 import importlib
 import os
@@ -9,10 +10,12 @@ import os
 import numpy as np
 import pytest
 
-from util import bits, golden_unary_case, tie_features
+from util import assert_same_as_reference, bits, golden_unary_case, tie_features
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 synth = importlib.import_module("lc-crf-slam_b200.synth")
+LATTICE_DIMS = (2, 3, 5)
+SLAM_SIZES = (2999, 3000, 3001, 3002, 20000)
 
 
 def test_golden_image_kat(oracle):
@@ -47,21 +50,24 @@ def test_golden_reference_vectors(oracle):
     assert np.array_equal(mp, g["slam_map"])
 
 
-@pytest.mark.parametrize("d", [2, 3, 5])
+def lattice_outputs(impl, f, xs):
+    """lattice of f and its filter of every x, by the oracle or the reference (the same API)"""
+    lat = impl.lattice(f)
+    out = {"V": np.array(lat["V"], np.int32), "offset": lat["offset"], "bary": lat["bary"], "nbr": lat["nbr"]}
+    for x in xs:
+        out["filter_L%d" % x.shape[1]] = impl.filter(lat, x)
+    impl.lattice_free(lat)
+    return out
+
+
+@pytest.mark.parametrize("d", LATTICE_DIMS)
 def test_lattice_vs_compiled_reference(oracle, ref, d):
     rng = np.random.default_rng(d)
     for N in (0, 1, 4, 5, 6, 7, 8, 257, 1000, 5003):
         f = tie_features(rng, N, d)
-        lo, lr = oracle.lattice(f), ref.lattice(f)
-        assert lo["V"] == lr["V"]
-        assert np.array_equal(lo["offset"], lr["offset"])
-        assert np.array_equal(bits(lo["bary"]), bits(lr["bary"]))
-        assert np.array_equal(lo["nbr"], lr["nbr"])
-        for L in (1, 2, 5):
-            x = rng.random((N, L)).astype(np.float32)
-            assert np.array_equal(bits(oracle.filter(lo, x)), bits(ref.filter(lr, x)))
-        oracle.lattice_free(lo)
-        ref.lattice_free(lr)
+        xs = [rng.random((N, L)).astype(np.float32) for L in (1, 2, 5)]
+        case = "lattice_d%d_n%d" % (d, N)
+        assert_same_as_reference(case, lattice_outputs(oracle, f, xs), ref.outputs(case, lambda r: lattice_outputs(r, f, xs)))
 
 
 def test_phantom_lanes(oracle):
@@ -75,19 +81,19 @@ def test_phantom_lanes(oracle):
     assert got == [3, 6, 6, 6, 3]
 
 
-@pytest.mark.parametrize("N", [2999, 3000, 3001, 3002, 20000])
+@pytest.mark.parametrize("N", SLAM_SIZES)
 def test_slam_crf_vs_compiled_reference(oracle, ref, N):
     from oracle.pyoracle import slam_params
     prm = slam_params(**synth.SLAM_PARAMS)
     fr = synth.slam_frame(N, seed=N)
     lab = oracle.rough_classify(fr.observs, fr.error, fr.depth, prm)
     assert 0 < lab.sum() < N
-    en = ref.label_energies(2, prm.confidence)
-    Qo, mo, V = oracle.slam_crf(fr.observs, fr.error, fr.kp2d, lab, en, prm)
-    Qr, mr = ref.slam_crf(fr.observs, fr.error, fr.kp2d, lab, prm)
-    assert np.array_equal(bits(Qo), bits(Qr))
-    assert np.array_equal(mo, mr)
-    assert 0 < mr.sum() < N  # non-trivial labelling
+    case = "slam_n%d" % N
+    want = ref.outputs(case, lambda r: dict(zip(("energies", "Q", "map"), (r.label_energies(2, prm.confidence),) +
+                                                r.slam_crf(fr.observs, fr.error, fr.kp2d, lab, prm))))
+    Qo, mo, _ = oracle.slam_crf(fr.observs, fr.error, fr.kp2d, lab, want["energies"], prm)
+    assert_same_as_reference(case, {"Q": Qo, "map": mo}, want)
+    assert 0 < mo.sum() < N  # non-trivial labelling
 
 
 def test_generic_labels_and_relax_vs_compiled_reference(oracle, ref):
@@ -99,9 +105,9 @@ def test_generic_labels_and_relax_vs_compiled_reference(oracle, ref):
         w = [3.0 + k for k in range(len(dims))]
         for relax in (1.0, 0.5):
             Qo, mo, _ = oracle.meanfield(unary, feats, w, 4, relax)
-            Qr, mr = ref.crf3d(L, feats, w, 4, unary=unary, relax=relax)
-            assert np.array_equal(bits(Qo), bits(Qr))
-            assert np.array_equal(mo, mr)
+            case = "generic_L%d_relax%g" % (L, relax)
+            want = ref.outputs(case, lambda r: dict(zip(("Q", "map"), r.crf3d(L, feats, w, 4, unary=unary, relax=relax))))
+            assert_same_as_reference(case, {"Q": Qo, "map": mo}, want)
 
 
 def test_fast_exp_properties(oracle):
@@ -230,10 +236,38 @@ def test_label_partition_restatement(oracle):
     assert d.size == 0 and s.size == 0
 
 
+def random_crf_case(oracle, ref, p):
+    """one case of the randomised sweep, p = [N, L, iters, relax, seed, conf (0: a random unary instead of labels), dims...]"""
+    N, L, iters, rs = int(p[0]), int(p[1]), int(p[2]), int(p[4])
+    relax, conf, dims = float(p[3]), float(p[5]), [int(d) for d in p[6:]]
+    rng = np.random.default_rng(rs)
+    feats = [tie_features(rng, N, d, float(rng.uniform(0.5, 8.0))) for d in dims]
+    w = rng.uniform(0.5, 30.0, len(dims)).astype(np.float32)
+    case = "random_%d_%d_%d_%s_%d_%s_%s" % (N, L, iters, relax, rs, conf, "-".join(map(str, dims)))
+    if conf:
+        lab = rng.integers(-1, L, N).astype(np.int16)
+        want = ref.outputs(case, lambda r: dict(zip(("params", "energies", "Q", "map"), (p, r.label_energies(L, conf)) +
+                                                    r.crf3d(L, feats, w, iters, label=lab, conf=conf, relax=relax))))
+        en = want["energies"]
+        unary = oracle.unary_from_label(lab, L, en[0], np.full(L, en[1], np.float32), np.full(L, en[2], np.float32))
+    else:
+        unary = (rng.random((N, L)) * 4).astype(np.float32)
+        want = ref.outputs(case, lambda r: dict(zip(("params", "Q", "map"), (p,) + r.crf3d(L, feats, w, iters, unary=unary, relax=relax))))
+    Qo, mo, _ = oracle.meanfield(unary, feats, w, iters, relax)
+    assert_same_as_reference(case, {"Q": Qo, "map": mo}, want)
+
+
 def test_random_crf_shapes_vs_compiled_reference(oracle, ref):
     """Randomised sweep (hypothesis, fixed seed): point counts incl. 0 and every N % 4 residue, labels, kernels,
     feature dimensions and scales, weights, iterations, relax, unary-from-label with unknown (-1) labels -- oracle
-    marginals and MAP bit-identical to the unmodified reference headers compiled in place."""
+    marginals and MAP bit-identical to the unmodified reference headers compiled in place.  Without them, the cases
+    this sweep drew when the reference outputs were stored are run against those outputs."""
+    if ref.live is None:
+        cases = ref.cases("random_")
+        assert cases
+        for case in cases:
+            random_crf_case(oracle, ref, ref.outputs(case, None)["params"])
+        return
     from hypothesis import given, settings, strategies as st, HealthCheck, seed
 
     @seed(20241)
@@ -246,23 +280,18 @@ def test_random_crf_shapes_vs_compiled_reference(oracle, ref):
         iters = data.draw(st.integers(1, 4), label="iters")
         relax = data.draw(st.sampled_from([1.0, 0.5, 0.3]), label="relax")
         rs = data.draw(st.integers(0, 2 ** 31 - 1), label="seed")
-        rng = np.random.default_rng(rs)
-        feats = [tie_features(rng, N, d, float(rng.uniform(0.5, 8.0))) for d in dims]
-        w = rng.uniform(0.5, 30.0, len(dims)).astype(np.float32)
-        if data.draw(st.booleans(), label="from_label"):
-            conf = float(data.draw(st.sampled_from([0.55, 0.7, 0.9]), label="conf"))
-            lab = rng.integers(-1, L, N).astype(np.int16)
-            en = ref.label_energies(L, conf)
-            unary = oracle.unary_from_label(lab, L, en[0], np.full(L, en[1], np.float32), np.full(L, en[2], np.float32))
-            Qr, mr = ref.crf3d(L, feats, w, iters, label=lab, conf=conf, relax=relax)
-        else:
-            unary = (rng.random((N, L)) * 4).astype(np.float32)
-            Qr, mr = ref.crf3d(L, feats, w, iters, unary=unary, relax=relax)
-        Qo, mo, _ = oracle.meanfield(unary, feats, w, iters, relax)
-        assert np.array_equal(bits(Qo), bits(Qr))
-        assert np.array_equal(mo, mr)
+        conf = float(data.draw(st.sampled_from([0.55, 0.7, 0.9]), label="conf")) if data.draw(st.booleans(), label="from_label") else 0.0
+        random_crf_case(oracle, ref, np.array([N, L, iters, relax, rs, conf] + dims, np.float64))
 
     run()
+
+
+def window_outputs(impl, f, x, L, io, oo, isz, osz):
+    """the reference's windowed filter (PermutohedralLatticeCPU::compute) of x on the lattice of f"""
+    lat = impl.lattice(f)
+    y = impl.filter_window(lat, x, L, io, oo, isz, osz)
+    impl.lattice_free(lat)
+    return {"y": y}
 
 
 def test_compute_window_is_zero_padding_plus_crop(oracle, ref):
@@ -272,16 +301,15 @@ def test_compute_window_is_zero_padding_plus_crop(oracle, ref):
     rng = np.random.default_rng(12)
     N, d = 1501, 2
     f = rng.normal(0, 2.0, (N, d)).astype(np.float32)
-    lr, lo = ref.lattice(f), oracle.lattice(f)
+    lo = oracle.lattice(f)
     for L, (io, oo, isz, osz) in ((1, (0, 0, -1, -1)), (2, (100, 0, 700, -1)), (3, (0, 37, -1, 900)), (21, (500, 1400, 1001, 101)),
                                   (2, (1500, 0, 1, 1)), (4, (0, 0, 0, -1))):
         n_in = N - io if isz == -1 else isz
         x = rng.normal(0, 1, (n_in, L)).astype(np.float32)
-        got = ref.filter_window(lr, x, L, io, oo, isz, osz)
         full = np.zeros((N, L), np.float32)
         full[io:io + n_in] = x
         n_out = N - oo if osz == -1 else osz
-        want = oracle.filter(lo, full)[oo:oo + n_out]
-        assert np.array_equal(got.view(np.int32), want.view(np.int32)), (L, io, oo, isz, osz)
-    ref.lattice_free(lr)
+        case = "window_L%d_%d_%d_%d_%d" % (L, io, oo, isz, osz)
+        want = ref.outputs(case, lambda r: window_outputs(r, f, x, L, io, oo, isz, osz))
+        assert_same_as_reference(case, {"y": oracle.filter(lo, full)[oo:oo + n_out]}, want)
     oracle.lattice_free(lo)

@@ -56,6 +56,58 @@ def tie_features(rng, N, d, scale=3.0):
     return f
 
 
+REF_SWEEP = "golden_ref_sweep.npz"  # in tests/golden/, written by tests/golden/make_golden_ref_sweep.py
+
+
+def fingerprint(a):
+    """sha256 of an array's dtype, shape and bits: how the larger reference outputs are stored"""
+    import hashlib
+    a = np.ascontiguousarray(a)
+    return "sha256:" + hashlib.sha256(("%s%s" % (a.dtype.str, a.shape)).encode() + a.tobytes()).hexdigest()
+
+
+class Reference:
+    """What the reference DenseCRF headers return on the inputs of tests/test_oracle.py: computed live by
+    oracle/_ref/libref.so where it was built (oracle/Makefile with the reference tree present), otherwise read from
+    tests/golden/golden_ref_sweep.npz."""
+
+    def __init__(self):
+        import os
+        from oracle.pyoracle import Ref
+        self.live = Ref() if Ref.available() else None
+        self.stored = {}
+        if self.live is None:
+            with np.load(os.path.join(os.path.dirname(__file__), "golden", REF_SWEEP)) as g:
+                for key in g.files:
+                    case, name = key.split("|")
+                    self.stored.setdefault(case, {})[name] = g[key]
+
+    def outputs(self, case, compute):
+        """{name: array} of one case; compute(Ref) evaluates it live.  A stored array may be a fingerprint."""
+        if self.live is not None:
+            return compute(self.live)
+        assert case in self.stored, "%s: no stored reference vectors (tests/golden/make_golden_ref_sweep.py)" % case
+        return self.stored[case]
+
+    def cases(self, prefix):
+        """the stored cases whose names start with `prefix`, in order"""
+        return sorted(c for c in self.stored if c.startswith(prefix))
+
+
+def assert_same_as_reference(case, got, want):
+    """every array of `got` (the oracle) bit for bit equal to the reference's array of the same name"""
+    for name, a in got.items():
+        a, w = np.asarray(a), np.asarray(want[name])
+        if w.dtype.kind == "U":
+            assert fingerprint(a) == str(w), "%s: %s differs from the reference" % (case, name)
+        else:
+            assert a.dtype == w.dtype and a.shape == w.shape, "%s: %s is %s%s, the reference's %s%s" % (
+                case, name, a.dtype, a.shape, w.dtype, w.shape)
+            u = np.dtype("u%d" % a.dtype.itemsize)
+            bad = int((np.ascontiguousarray(a).reshape(-1).view(u) != np.ascontiguousarray(w).reshape(-1).view(u)).sum())
+            assert bad == 0, "%s: %d of %d values of %s differ from the reference in bits" % (case, bad, a.size, name)
+
+
 def golden_unary_case(name):
     """One case of tests/golden/golden_unary.npz (made by tests/golden/make_golden_unary.py with the real cv2.gemm):
     returns (MapSnapshot, observs, error, depth)."""
