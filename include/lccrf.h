@@ -282,6 +282,42 @@ int lccrf_frames_debug_counters(lccrf_frames *fr, int k, int *out8);
 /* algorithmic bytes of one lccrf_frames_run by the SURVEY 8(d) formulas with the actual V (valid after a run) */
 int lccrf_frames_algorithmic_bytes(lccrf_frames *fr, double *total, double *per_iteration, double *unary);
 
+/* ---------------------------------------------------------------- batched images --------- */
+/* B independent full-image CRFs in one launch sequence: for every image
+ *   DenseCRFCPU<M> crf(W*H); crf.setUnaryEnergy(...) or setUnaryEnergyFromLabel(...);
+ *   crf.addPairwiseEnergy(PottsPotentialCPU<M,F>::FromImage(W, H, w, posdev, img, featuredev)) for each kernel;
+ *   crf.inference(n_iterations, true, relax)
+ *   (Thirdparty/DenseCRF/examples/example_cpu.cpp:80-102).  Image sizes, labels and kernels are fixed at create; each
+ * run rebuilds the lattices from the current pixels.  Marginals and MAP labels are bit-identical, image by image, to the
+ * lccrf_crf path (lccrf_crf_add_potts_image) on the same inputs. */
+typedef struct lccrf_images lccrf_images;
+/* one Potts potential of PottsPotentialCPU<M,F>::FromImage (pairwise_cpu.h:34-50) */
+typedef struct lccrf_image_kernel {
+    int F;              /* 2: Gaussian on (x/posdev, y/posdev); C + 2: bilateral, adds the C image channels / featuredev */
+    float w, posdev, featuredev;
+} lccrf_image_kernel;
+/* B images; image b is W[b] x H[b] pixels, row-major (pixel index y*W[b] + x, as pairwise_cpu.h:41-44), images
+ * concatenated in order (NT = sum of W[b]*H[b] pixels).  C channels per pixel (0 when every kernel has F == 2), L labels,
+ * K kernels in the order addPairwiseEnergy would attach them.  At most 2^22 pixels per image. */
+int  lccrf_images_create(lccrf_ctx *ctx, int B, const int *W, const int *H, int C, int L, int K,
+                         const lccrf_image_kernel *kernels, lccrf_images **out);
+void lccrf_images_destroy(lccrf_images *im);
+/* img [NT*C] u8 (img_is_u8) or f32, NULL when C == 0 or no kernel is bilateral.  unary [NT*L]: setUnaryEnergy
+ * (densecrf3d.h:41-43).  The arrays have been read when the call returns (it synchronises). */
+int  lccrf_images_set_inputs(lccrf_images *im, const void *img, int img_is_u8, const float *unary);
+/* ... or setUnaryEnergyFromLabel (densecrf3d.h:108-130): label [NT] in [-1, L), tables as lccrf_crf_set_unary_from_label.
+ * Labels are checked on the device: one outside [-1, L) makes lccrf_images_get_outputs return LCCRF_ERR_ARG. */
+int  lccrf_images_set_inputs_from_label(lccrf_images *im, const void *img, int img_is_u8, const short *label,
+                                        float u_energy, const float *n_energies, const float *p_energies);
+/* inference(n_iterations, true, relax) for every image, asynchronous on the context's stream.  With option "graphs" the
+ * second run of the same (n_iterations, relax, input mode) captures a CUDA graph and later runs replay it. */
+int  lccrf_images_run(lccrf_images *im, int n_iterations, float relax);
+/* synchronises; map [NT], prob [NT*L], either may be NULL; reports errors raised on the device (key range, labels).
+ * LCCRF_ERR_STATE before the first run.  The object stays usable after an error. */
+int  lccrf_images_get_outputs(lccrf_images *im, short *map, float *prob);
+/* M_ of every lattice after a run: V [B*K], image-major (diagnostics / tests); synchronises */
+int  lccrf_images_vertices(lccrf_images *im, int *V);
+
 /* ---------------------------------------------------------------- device-resident map ----- */
 /* In the reference the observation lists, keyframe poses and keypoints are persistent MAP state that tracking only reads
  * (Tracking::ComputeMapPointErrAndObserv, src/Tracking.cc:1803-1839) and local mapping mutates a little per keyframe.

@@ -52,10 +52,16 @@ class SlamParams(C.Structure):
         return p
 
 
+class ImageKernel(C.Structure):
+    """lccrf_image_kernel: one PottsPotentialCPU<M,F>::FromImage potential (F = 2: Gaussian, F = C + 2: bilateral)."""
+    _fields_ = [("F", C.c_int), ("w", C.c_float), ("posdev", C.c_float), ("featuredev", C.c_float)]
+
+
 _fp = C.POINTER(C.c_float)
 _ip = C.POINTER(C.c_int)
 _sp = C.POINTER(C.c_short)
 _vp = C.c_void_p
+_byref = C.byref  # Images takes a parameter named C
 
 # every symbol include/lccrf.h declares: (restype, argtypes)
 SYMBOLS = {
@@ -115,6 +121,13 @@ SYMBOLS = {
     "lccrf_frames_get_debug": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "lccrf_frames_debug_counters": (C.c_int, [_vp, C.c_int, _vp]),
     "lccrf_frames_algorithmic_bytes": (C.c_int, [_vp, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double)]),
+    "lccrf_images_create": (C.c_int, [_vp, C.c_int, _vp, _vp, C.c_int, C.c_int, C.c_int, C.POINTER(ImageKernel), C.POINTER(_vp)]),
+    "lccrf_images_destroy": (None, [_vp]),
+    "lccrf_images_set_inputs": (C.c_int, [_vp, _vp, C.c_int, _vp]),
+    "lccrf_images_set_inputs_from_label": (C.c_int, [_vp, _vp, C.c_int, _vp, C.c_float, _vp, _vp]),
+    "lccrf_images_run": (C.c_int, [_vp, C.c_int, C.c_float]),
+    "lccrf_images_get_outputs": (C.c_int, [_vp, _vp, _vp]),
+    "lccrf_images_vertices": (C.c_int, [_vp, _vp]),
     "lccrf_map_create": (C.c_int, [_vp, C.c_int, C.POINTER(_vp)]),
     "lccrf_map_destroy": (None, [_vp]),
     "lccrf_map_apply": (C.c_int, [_vp, _vp]),
@@ -707,6 +720,81 @@ class Frames:
     def close(self):
         if getattr(self, "h", None):
             self.ctx.lib.lccrf_frames_destroy(self.h)
+            self.h = None
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+class Images:
+    """lccrf_images: B full-image DenseCRFs (DenseCRFCPU<M> + PottsPotentialCPU<M,F>::FromImage) in one launch sequence.
+
+    sizes: [(W, H), ...] per image; kernels: [(F, w, posdev, featuredev), ...] in addPairwiseEnergy order (F = 2 Gaussian,
+    F = C + 2 bilateral); C: channels per pixel.  Arrays are concatenated over the images in order."""
+
+    def __init__(self, ctx: Context, sizes, L: int, kernels, C: int = 3):
+        self.ctx, self.L, self.C = ctx, int(L), int(C)
+        wh = np.asarray(sizes, dtype=np.int32).reshape(-1, 2)
+        self.W, self.H = np.ascontiguousarray(wh[:, 0]), np.ascontiguousarray(wh[:, 1])
+        self.B = int(wh.shape[0])
+        self.ptr = np.zeros(self.B + 1, dtype=np.int64)
+        np.cumsum(self.W.astype(np.int64) * self.H, out=self.ptr[1:])
+        self.NT = int(self.ptr[-1])
+        self.K = len(kernels)
+        ks = (ImageKernel * max(self.K, 1))(*[ImageKernel(int(F), w, posdev, fd) for F, w, posdev, fd in kernels])
+        h = _vp()
+        ctx._check(ctx.lib.lccrf_images_create(ctx.h, self.B, _ptr(self.W), _ptr(self.H), self.C, self.L, self.K, ks, _byref(h)))
+        self.h = h
+        ctx._children.add(self)
+
+    def _cat(self, a, dtype=None):
+        if isinstance(a, (list, tuple)):
+            a = np.concatenate([np.asarray(x).reshape(-1) for x in a]) if a else np.zeros(0, dtype or np.float32)
+        return None if a is None else np.ascontiguousarray(a, dtype=dtype)
+
+    def set_inputs(self, img, unary=None, label=None, energies=None):
+        """img: [NT, C] (or a list per image) uint8 or float32, None without bilateral kernels.  Either unary [NT, L]
+        (setUnaryEnergy) or label [NT] with energies = {u, n, p} of label_energies, or (u, n_en[L], p_en[L])."""
+        img = self._cat(img)
+        u8 = img is None or img.dtype == np.uint8
+        if img is not None and not u8:
+            img = np.ascontiguousarray(img, dtype=np.float32)
+        if unary is not None:
+            u = self._cat(unary, np.float32)
+            self.ctx._check(self.ctx.lib.lccrf_images_set_inputs(self.h, _ptr(img), int(u8), _ptr(u)))
+            return
+        lab = self._cat(label, np.int16)
+        if energies is None or len(energies) == 3 and np.ndim(energies[1]) == 0:
+            e = label_energies(self.L, 0.5) if energies is None else np.asarray(energies, np.float32)
+            u_en, n_en, p_en = float(e[0]), np.full(self.L, e[1], np.float32), np.full(self.L, e[2], np.float32)
+        else:
+            u_en, n_en, p_en = float(energies[0]), _arr(energies[1], np.float32), _arr(energies[2], np.float32)
+        self.ctx._check(self.ctx.lib.lccrf_images_set_inputs_from_label(self.h, _ptr(img), int(u8), _ptr(lab), u_en,
+                                                                        _ptr(n_en), _ptr(p_en)))
+
+    def run(self, T: int, relax: float = 1.0):
+        self.ctx._check(self.ctx.lib.lccrf_images_run(self.h, int(T), float(relax)))
+
+    def get_outputs(self, want_prob=True, map_out=None, prob_out=None):
+        """(map [NT], prob [NT, L] or None, [(map_b, prob_b), ...] views per image); synchronises"""
+        mp = np.empty(self.NT, dtype=np.int16) if map_out is None else map_out
+        pr = (np.empty((self.NT, self.L), dtype=np.float32) if prob_out is None else prob_out) if want_prob else None
+        self.ctx._check(self.ctx.lib.lccrf_images_get_outputs(self.h, _ptr(mp), _ptr(pr)))
+        split = [(mp[a:b], None if pr is None else pr[a:b]) for a, b in zip(self.ptr[:-1], self.ptr[1:])]
+        return mp, pr, split
+
+    def vertices(self) -> np.ndarray:
+        """[B, K] lattice vertex counts (M_) of the last run"""
+        V = np.zeros((self.B, self.K), dtype=np.int32)
+        self.ctx._check(self.ctx.lib.lccrf_images_vertices(self.h, _ptr(V)))
+        return V
+
+    def close(self):
+        if getattr(self, "h", None):
+            self.ctx.lib.lccrf_images_destroy(self.h)
             self.h = None
 
     def __del__(self):

@@ -94,17 +94,18 @@ static void scratch_release(Ctx *ctx, Ctx::Scratch &s, bool pinned) {
 }
 
 // device status word -> error code (bits: 1 lattice key range, 2 index out of range, 4 visible point without
-// observations, 8 a point twice in one delta list, 16 observation pool exhausted)
+// observations, 8 a point twice in one delta list, 16 observation pool exhausted, 32 label outside [-1, L))
 static int decode_status(int st) {
     if (st & 1) return fail(LCCRF_ERR_RANGE, "lattice key outside the reference's short range (permutohedral_cpu.h:373)");
     if (st & 2) return fail(LCCRF_ERR_ARG, "an observation, keyframe, feature or point index is outside its table");
     if (st & 4) return fail(LCCRF_ERR_ARG, "a visible map point has no observations (Tracking.cc:1858 drops such points before the CRF)");
     if (st & 8) return fail(LCCRF_ERR_ARG, "a point appears twice in one list of a map delta (split it over several deltas)");
     if (st & 16) return fail(LCCRF_ERR_STATE, "observation pool exhausted: call lccrf_map_reserve_observations and repeat the step");
+    if (st & 32) return fail(LCCRF_ERR_ARG, "a label is outside [-1, L)");
     return LCCRF_OK;
 }
 
-static int check_status(Ctx *ctx) {  // synchronises
+int check_status(Ctx *ctx) {  // synchronises
     LCCRF_CUDA(cudaMemcpyAsync(ctx->h_status, ctx->d_status, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
     LCCRF_CUDA(cudaStreamSynchronize(ctx->stream));
     if (*ctx->h_status) {
@@ -114,7 +115,7 @@ static int check_status(Ctx *ctx) {  // synchronises
     return LCCRF_OK;
 }
 
-static int batch_init(Ctx *ctx, Batch &b, int B, const int *prob_ptr, int L, bool with_state) {
+int batch_init(Ctx *ctx, Batch &b, int B, const int *prob_ptr, int L, bool with_state) {
     b.ctx = ctx;
     b.B = B;
     b.L = L;
@@ -128,6 +129,7 @@ static int batch_init(Ctx *ctx, Batch &b, int B, const int *prob_ptr, int L, boo
     }
     if (b.maxN > (1 << 22)) return fail(LCCRF_ERR_ARG, "more than 2^22 points in one problem (fixed-point splat range)");
     b.NT = b.h_prob_ptr[B];
+    b.fused_blur = B >= 2 || b.maxN <= kFusedBlurMaxN;
     LCCRF_TRY(dev_alloc(ctx, (void **)&b.prob_ptr, (size_t)(B + 1) * sizeof(int)));
     LCCRF_CUDA(cudaMemcpyAsync(b.prob_ptr, b.h_prob_ptr.data(), (size_t)(B + 1) * sizeof(int), cudaMemcpyHostToDevice,
                                ctx->stream));
@@ -143,7 +145,7 @@ static int batch_init(Ctx *ctx, Batch &b, int B, const int *prob_ptr, int L, boo
     return LCCRF_OK;
 }
 
-static void batch_release(Ctx *ctx, Batch &b) {
+void batch_release(Ctx *ctx, Batch &b) {
     for (auto *ls : b.lat) lattice_set_destroy(ctx, ls);
     b.lat.clear();
     dev_free(ctx, b.prob_ptr);
@@ -155,6 +157,53 @@ static void batch_release(Ctx *ctx, Batch &b) {
     b.prob_ptr = nullptr;
     b.unary = b.cur = b.next = b.tmp = nullptr;
     b.map = nullptr;
+}
+
+void graph_drop(GraphReplay &g) {
+    if (g.exec) cudaGraphExecDestroy(g.exec);
+    g.exec = nullptr;
+    g.same_shape_runs = 0;
+}
+
+bool graph_will_capture(const Ctx *ctx, const GraphReplay &g) {
+    return ctx->opt_graphs && !ctx->opt_profile && !g.exec && g.same_shape_runs > 0;
+}
+
+int graph_run(Ctx *ctx, GraphReplay &g, const std::function<int()> &enqueue) {
+    if (!ctx->opt_graphs || ctx->opt_profile) return enqueue();
+    if (g.exec && g.gen != ctx->scratch_gen) graph_drop(g);  // a scratch buffer moved since capture
+    if (!g.exec && g.same_shape_runs == 0) {
+        // A new shape: plain launches, no synchronisation.  A graph is only worth capturing for a shape that repeats,
+        // so the capture waits for the second run of the same shape.
+        g.same_shape_runs = 1;
+        return enqueue();
+    }
+    if (!g.exec) {
+        // make sure every scratch buffer has its final size before capture (no allocation inside the graph)
+        const uint64_t l0 = ctx->launches;
+        LCCRF_TRY(enqueue());
+        LCCRF_CUDA(cudaStreamSynchronize(ctx->stream));
+        const uint64_t per_run = ctx->launches - l0;
+        cudaGraph_t cg = nullptr;
+        LCCRF_CUDA(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
+        int rc = enqueue();
+        cudaError_t e = cudaStreamEndCapture(ctx->stream, &cg);
+        ctx->launches -= per_run;  // the capture pass launched nothing
+        if (rc != LCCRF_OK) {
+            if (cg) cudaGraphDestroy(cg);
+            return rc;
+        }
+        if (e != cudaSuccess) return fail(LCCRF_ERR_CUDA, std::string("graph capture: ") + cudaGetErrorString(e));
+        e = cudaGraphInstantiate(&g.exec, cg, 0);
+        cudaGraphDestroy(cg);
+        if (e != cudaSuccess) return fail(LCCRF_ERR_CUDA, std::string("graph instantiate: ") + cudaGetErrorString(e));
+        g.launches = per_run;
+        g.gen = ctx->scratch_gen;
+        return LCCRF_OK;  // the warm-up pass above already produced this call's results
+    }
+    LCCRF_CUDA(cudaGraphLaunch(g.exec, ctx->stream));
+    ctx->launches += g.launches;
+    return LCCRF_OK;
 }
 
 }  // namespace lccrf
@@ -180,11 +229,7 @@ struct PhaseTimer {
     }
 };
 
-// ------------------------------------------------------------------ opaque handle types
-struct lccrf_ctx {
-    Ctx c;
-};
-
+// ------------------------------------------------------------------ opaque handle types (lccrf_ctx: engine.cuh)
 struct lccrf_lattice {
     Ctx *ctx = nullptr;
     Batch b;
@@ -251,9 +296,8 @@ struct FrameInputs {
     const int *part_fid = nullptr;
     int *part_dyn_ptr = nullptr, *part_dyn = nullptr, *part_stat_ptr = nullptr, *part_stat = nullptr;
     bool have_inputs = false;
-    cudaGraphExec_t graph = nullptr;
-    int same_shape_runs = 0;  // runs since the launch sequence of this slot last changed shape (a graph is captured on the 2nd)
-    uint64_t graph_launches = 0, graph_gen = 0, kp_gen = 0;
+    GraphReplay graph;
+    uint64_t kp_gen = 0;
     cudaEvent_t up_done = nullptr, run_done = nullptr, out_done = nullptr;
     int *h_status = nullptr;  // pinned copy of the device status word taken after this slot's run
     bool in_flight = false;
@@ -1059,14 +1103,8 @@ int lccrf_frames_create(lccrf_ctx *h, int B, const int *prob_ptr, const lccrf_sl
     return LCCRF_OK;
 }
 
-static void frame_inputs_drop_graph(FrameInputs &in) {
-    if (in.graph) cudaGraphExecDestroy(in.graph);
-    in.graph = nullptr;
-    in.same_shape_runs = 0;
-}
-
 static void frame_inputs_release(Ctx *ctx, FrameInputs &in) {
-    frame_inputs_drop_graph(in);
+    graph_drop(in.graph);
     dev_free(ctx, in.observs);
     dev_free(ctx, in.error);
     dev_free(ctx, in.depth);
@@ -1129,7 +1167,7 @@ static int order_copies_after_alloc(Ctx *ctx, FrameInputs &in, cudaStream_t st) 
 static int frames_upload_prior(lccrf_frames *fr, FrameInputs &in, cudaStream_t st) {
     Ctx *ctx = fr->ctx;
     const bool use = in.h_p4 != nullptr && fr->b.NT > 0, use_has = use && in.h_p4_has != nullptr;
-    if (use != in.use_p4 || use_has != in.use_p4_has) frame_inputs_drop_graph(in);  // the classifier's arguments change
+    if (use != in.use_p4 || use_has != in.use_p4_has) graph_drop(in.graph);  // the classifier's arguments change
     in.use_p4 = use;
     in.use_p4_has = use_has;
     if (!use) return LCCRF_OK;
@@ -1137,7 +1175,7 @@ static int frames_upload_prior(lccrf_frames *fr, FrameInputs &in, cudaStream_t s
     if (!in.p4) {
         LCCRF_TRY(dev_alloc(ctx, (void **)&in.p4, (size_t)fr->b.NT * sizeof(double)));
         LCCRF_TRY(dev_alloc(ctx, (void **)&in.p4_has, (size_t)fr->b.B));
-        frame_inputs_drop_graph(in);
+        graph_drop(in.graph);
         fresh = true;
     }
     if (fresh) LCCRF_TRY(order_copies_after_alloc(ctx, in, st));
@@ -1157,16 +1195,16 @@ static int frames_upload_direct(lccrf_frames *fr, FrameInputs &in, cudaStream_t 
         LCCRF_TRY(dev_alloc(ctx, (void **)&in.observs, m * 4));
         LCCRF_TRY(dev_alloc(ctx, (void **)&in.error, m * 4));
         LCCRF_TRY(dev_alloc(ctx, (void **)&in.depth, m * 4));
-        frame_inputs_drop_graph(in);
+        graph_drop(in.graph);
         fresh = true;
     }
     if (!in.kp2d) {
         LCCRF_TRY(dev_alloc(ctx, (void **)&in.kp2d, (n ? n : 1) * 8));
-        frame_inputs_drop_graph(in);
+        graph_drop(in.graph);
         fresh = true;
     }
     if (fresh) LCCRF_TRY(order_copies_after_alloc(ctx, in, st));
-    if (in.from_map) frame_inputs_drop_graph(in);
+    if (in.from_map) graph_drop(in.graph);
     in.from_map = false;
     in.visible = false;
     LCCRF_TRY(frames_upload_prior(fr, in, st));
@@ -1264,7 +1302,7 @@ static int frames_upload_map(lccrf_frames *fr, FrameInputs &in, cudaStream_t st,
     if (in.nKF != nKF || in.nnz != nnz || !in.from_map || in.visible || in.have_kf_ptr != (kf_ptr != nullptr)) regraph = true;
     in.visible = false;
     if (regraph) {
-        frame_inputs_drop_graph(in);
+        graph_drop(in.graph);
         LCCRF_TRY(order_copies_after_alloc(ctx, in, st));  // every (re)allocation above sets regraph
     }
     in.nKF = nKF;
@@ -1373,51 +1411,12 @@ static int frames_run_slot(lccrf_frames *fr, FrameInputs &in) {
         LCCRF_TRY(map_end_async_mut(in.map));
     }
     if (in.visible) LCCRF_TRY(map_begin_main_access(in.map));
-    if (!ctx->opt_graphs || ctx->opt_profile) {
-        LCCRF_TRY(frames_enqueue(fr, in));
-        fr->ran = true;
-        return LCCRF_OK;
-    }
-    if (in.graph && in.graph_gen != ctx->scratch_gen) frame_inputs_drop_graph(in);  // a scratch buffer moved since capture
-    if (in.indexed && in.kp_gen != fr->kp_gen) {  // the keypoint table moved (keyframes inserted) since this slot was captured
-        frame_inputs_drop_graph(in);
+    if (ctx->opt_graphs && !ctx->opt_profile && in.indexed && in.kp_gen != fr->kp_gen) {
+        // the keypoint table moved (keyframes inserted) since this slot was captured
+        graph_drop(in.graph);
         in.kp_gen = fr->kp_gen;
     }
-    if (!in.graph && in.same_shape_runs == 0) {
-        // A new shape (observation count, keyframe count, camera model, buffers): plain launches, no synchronisation.
-        // In live SLAM these change every frame; a graph is only worth capturing for a shape that repeats (replay), so
-        // the capture waits for the second run of the same shape.
-        in.same_shape_runs = 1;
-        LCCRF_TRY(frames_enqueue(fr, in));
-        fr->ran = true;
-        return LCCRF_OK;
-    }
-    if (!in.graph) {
-        // make sure every scratch buffer has its final size before capture (no allocation inside the graph)
-        const uint64_t l0 = ctx->launches;
-        LCCRF_TRY(frames_enqueue(fr, in));
-        LCCRF_CUDA(cudaStreamSynchronize(ctx->stream));
-        const uint64_t per_run = ctx->launches - l0;
-        cudaGraph_t g = nullptr;
-        LCCRF_CUDA(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
-        int rc = frames_enqueue(fr, in);
-        cudaError_t e = cudaStreamEndCapture(ctx->stream, &g);
-        ctx->launches -= per_run;  // the capture pass launched nothing
-        if (rc != LCCRF_OK) {
-            if (g) cudaGraphDestroy(g);
-            return rc;
-        }
-        if (e != cudaSuccess) return fail(LCCRF_ERR_CUDA, std::string("graph capture: ") + cudaGetErrorString(e));
-        e = cudaGraphInstantiate(&in.graph, g, 0);
-        cudaGraphDestroy(g);
-        if (e != cudaSuccess) return fail(LCCRF_ERR_CUDA, std::string("graph instantiate: ") + cudaGetErrorString(e));
-        in.graph_launches = per_run;
-        in.graph_gen = ctx->scratch_gen;
-        fr->ran = true;
-        return LCCRF_OK;  // the warm-up pass above already produced this call's results
-    }
-    LCCRF_CUDA(cudaGraphLaunch(in.graph, ctx->stream));
-    ctx->launches += in.graph_launches;
+    LCCRF_TRY(graph_run(ctx, in.graph, [&] { return frames_enqueue(fr, in); }));
     fr->ran = true;
     return LCCRF_OK;
 }
@@ -1472,7 +1471,7 @@ static int frames_submit_epilogue(lccrf_frames *fr, int slot, FrameInputs &in, s
     Ctx *ctx = fr->ctx;
     LCCRF_CUDA(cudaEventRecord(in.up_done, ctx->copy_stream));
     LCCRF_CUDA(cudaStreamWaitEvent(ctx->stream, in.up_done, 0));
-    if (!in.graph && in.same_shape_runs > 0 && ctx->opt_graphs && !ctx->opt_profile) {
+    if (graph_will_capture(ctx, in.graph)) {
         // the capture pass synchronises; make sure the upload has landed first
         LCCRF_CUDA(cudaStreamSynchronize(ctx->copy_stream));
     }
@@ -2042,7 +2041,7 @@ static int frames_upload_visible(lccrf_frames *fr, FrameInputs &in, cudaStream_t
         regraph = fresh = true;
     }
     if (!in.visible || in.map != m || in.have_kf_ptr != (kf_ptr != nullptr)) regraph = true;
-    if (regraph) frame_inputs_drop_graph(in);
+    if (regraph) graph_drop(in.graph);
     if (fresh) LCCRF_TRY(order_copies_after_alloc(ctx, in, st));
     in.visible = true;
     in.from_map = true;

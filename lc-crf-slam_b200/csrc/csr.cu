@@ -370,21 +370,31 @@ int csr_create(Ctx *ctx, const Batch &b, LatticeSet *ls) {
     std::vector<int> chunk_prob, chunk_s0, chunk_s1, prob_chunk0(b.B + 1);
     std::vector<long long> chunk_tbl;
     long long tbl = 0;
-    for (int i = 0; i < b.B; i++) {
-        prob_chunk0[i] = (int)chunk_prob.size();
-        const int p0 = b.h_prob_ptr[i], p1 = b.h_prob_ptr[i + 1];
-        const long long stride = ((long long)(p1 - p0) + 1) * D;  // worst-case vertex count of the problem
-        // the count table is chunks x vertices: image-scale problems (millions of points) take coarser chunks so
-        // that one problem's table stays below 2^30 entries
-        long long cpts = kCsrChunkPoints;
-        while (((long long)(p1 - p0) + cpts - 1) / cpts * stride > (1ll << 30)) cpts *= 2;
-        for (long long c = p0; c < p1; c += cpts) {
-            chunk_prob.push_back(i);
-            chunk_s0.push_back((int)(c * D));
-            chunk_s1.push_back((int)((c + cpts < p1 ? c + cpts : p1) * D));
-            chunk_tbl.push_back(tbl);
-            tbl += stride;
+    // The chunk size sets the parallelism of the sort, not its result (rows keep point order either way).  A batch of
+    // many image-sized problems whose tables together exceed 2^31 entries takes coarser chunks in every problem.
+    for (long long min_cpts = kCsrChunkPoints;; min_cpts *= 2) {
+        chunk_prob.clear();
+        chunk_s0.clear();
+        chunk_s1.clear();
+        chunk_tbl.clear();
+        tbl = 0;
+        for (int i = 0; i < b.B; i++) {
+            prob_chunk0[i] = (int)chunk_prob.size();
+            const int p0 = b.h_prob_ptr[i], p1 = b.h_prob_ptr[i + 1];
+            const long long stride = ((long long)(p1 - p0) + 1) * D;  // worst-case vertex count of the problem
+            // the count table is chunks x vertices: image-scale problems (millions of points) take coarser chunks so
+            // that one problem's table stays below 2^30 entries
+            long long cpts = min_cpts;
+            while (((long long)(p1 - p0) + cpts - 1) / cpts * stride > (1ll << 30)) cpts *= 2;
+            for (long long c = p0; c < p1; c += cpts) {
+                chunk_prob.push_back(i);
+                chunk_s0.push_back((int)(c * D));
+                chunk_s1.push_back((int)((c + cpts < p1 ? c + cpts : p1) * D));
+                chunk_tbl.push_back(tbl);
+                tbl += stride;
+            }
         }
+        if (tbl <= (1ll << 31) - 1 || min_cpts > b.maxN) break;
     }
     prob_chunk0[b.B] = (int)chunk_prob.size();
     ls->csr_chunks = (int)chunk_prob.size();

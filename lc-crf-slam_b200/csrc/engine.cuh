@@ -5,6 +5,7 @@
 #pragma once
 
 #include <cstddef>
+#include <functional>
 #include <vector>
 
 #include "common.cuh"
@@ -73,6 +74,9 @@ struct Batch {
     std::vector<int> h_prob_ptr;  // host copy
     int *prob_ptr = nullptr;      // [B+1] device
     int maxN = 0;
+    // blur of every filter call: true = k_blur_fused, one CTA per problem runs all D passes out of shared memory;
+    // false = element-parallel passes (k_blur_bulk / k_blur_vec) over the vertices of all problems, one launch per pass
+    bool fused_blur = false;
     std::vector<LatticeSet *> lat;  // K potentials
     float *unary = nullptr, *cur = nullptr, *next = nullptr, *tmp = nullptr;  // [NT*L]
     short *map = nullptr;                                                      // [NT]
@@ -132,6 +136,28 @@ struct Ctx {
 };
 
 int ctx_scratch(Ctx *ctx, Ctx::Scratch &s, size_t bytes, bool pinned = false);
+
+// batches (api.cu).  batch_init sets fused_blur = B >= 2 || maxN <= kFusedBlurMaxN (the rule of lccrf_crf and lccrf_frames);
+// a caller with another rule overwrites it before the first filter call.
+constexpr int kFusedBlurMaxN = 32768;
+int batch_init(Ctx *ctx, Batch &b, int B, const int *prob_ptr, int L, bool with_state);
+void batch_release(Ctx *ctx, Batch &b);
+// device status word: read (synchronises), clear, and turn the first error it holds into a return code
+int check_status(Ctx *ctx);
+
+// CUDA-graph replay of a launch sequence whose shape repeats.  The first run of a shape launches plainly; the second
+// runs once more uncaptured (every scratch buffer reaches its final size) and captures; later runs replay.  A caller
+// whose launch arguments change calls graph_drop, which makes the next run the first of a new shape.
+struct GraphReplay {
+    cudaGraphExec_t exec = nullptr;
+    int same_shape_runs = 0;  // runs since the launch sequence last changed shape (a graph is captured on the 2nd)
+    uint64_t launches = 0;    // kernels one replay stands for
+    uint64_t gen = 0;         // Ctx::scratch_gen at capture
+};
+void graph_drop(GraphReplay &g);
+// true when the next graph_run will capture (it synchronises the context's stream)
+bool graph_will_capture(const Ctx *ctx, const GraphReplay &g);
+int graph_run(Ctx *ctx, GraphReplay &g, const std::function<int()> &enqueue);
 
 // RAII bracket around one kernel launch: counts it and, in profile mode, times it with CUDA events
 // recorded on the launching stream.
@@ -314,8 +340,9 @@ int filter_splat_blur(Ctx *ctx, const Batch &b, LatticeSet *ls, const float *in_
 int filter_full(Ctx *ctx, const Batch &b, LatticeSet *ls, float *out_dev, const float *in_dev, int L);
 int potts_norm(Ctx *ctx, const Batch &b, LatticeSet *ls);
 // mean field (meanfield.cu)
+// status (optional): a label outside [-1, L) sets 32 in the device status word and is read as unknown (u_energy)
 int mf_unary_from_label(Ctx *ctx, float *unary, const short *label_dev, int NT, int L, float u_energy,
-                        const float *n_en, const float *p_en);
+                        const float *n_en, const float *p_en, int *status = nullptr);
 int mf_exp_and_normalize(Ctx *ctx, float *out, const float *in, int NT, int L, float scale, float relax);
 int mf_start(Ctx *ctx, Batch &b);
 int mf_step(Ctx *ctx, Batch &b, float relax);
@@ -334,6 +361,10 @@ int feat_div2(Ctx *ctx, float *feat, const float *a, int stride_a, float sa, con
               float sb, int N);
 int feat_image(Ctx *ctx, float *feat, int W, int H, int F, float posdev, const void *img_dev, int is_u8,
                float featuredev);
+// the features of feat_image for every image of a batch in one launch: image b is pixels [prob_ptr[b], prob_ptr[b+1]),
+// width[b] pixels wide (device arrays [B+1] / [B]); img_dev [NT*(F-2)]
+int feat_image_batch(Ctx *ctx, float *feat, int NT, int B, const int *prob_ptr, const int *width, int F, float posdev,
+                     const void *img_dev, int is_u8, float featuredev);
 int unary_pack_kf(Ctx *ctx, void *kf_packed /*nKF*80 B*/, const float *pose, const float *intr, const float *bnd, int nKF);
 int unary_map_points_packed(Ctx *ctx, int N, int nKF, const float *xyz, const int *obs_ptr, const void *obs_kf,
                             int obs_kf_bytes, const float *obs_uv, const void *kf_packed, float *observs, float *error, float *depth,
@@ -370,3 +401,8 @@ int bf_match(Ctx *ctx, int B, int NQ, int max_nq, int max_nt, const int *q_ptr, 
              int *n_match);
 
 }  // namespace lccrf
+
+// opaque handle of include/lccrf.h (its entry points are spread over api.cu and images.cu)
+struct lccrf_ctx {
+    lccrf::Ctx c;
+};

@@ -1499,7 +1499,7 @@ int filter_splat_blur(Ctx *ctx, const Batch &b, LatticeSet *ls, const float *in_
         LCCRF_CUDA(cudaEventRecord(ctx->ev_sub_join[ctx->branch], ctx->sub_stream[ctx->branch]));
         LCCRF_CUDA(cudaStreamWaitEvent(st, ctx->ev_sub_join[ctx->branch], 0));
     }
-    if (b.B >= 2 || b.maxN <= 32768) {  // one CTA per problem runs all D passes
+    if (b.fused_blur) {  // one CTA per problem runs all D passes
         LCCRF_TRY(ensure_dyn_smem(ctx, k_blur_fused, kBlurFusedBytes + 16));
         LCCRF_KERNEL(ctx, "k_blur_fused");
         k_blur_fused<<<b.B, 1024, kBlurFusedBytes + 16, st>>>(ls->nbr, ls->Vcap, ls->vbase, src, dst, L, D);

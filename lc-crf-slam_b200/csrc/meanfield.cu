@@ -103,11 +103,15 @@ k_exp_normalize(float *__restrict__ out, const float *__restrict__ in, int NT, i
 
 __global__ void __launch_bounds__(kThreads)
 k_unary_from_label(float *__restrict__ unary, const short *__restrict__ label, int NT, int L, float u_energy,
-                   const float *__restrict__ n_en, const float *__restrict__ p_en) {
+                   const float *__restrict__ n_en, const float *__restrict__ p_en, int *__restrict__ status) {
     const long long t = (long long)blockIdx.x * kThreads + threadIdx.x;
     if (t >= (long long)NT * L) return;
     const int i = (int)(t / L), m = (int)(t - (long long)i * L);
-    const int lab = label[i];
+    int lab = label[i];
+    if (status && (lab < -1 || lab >= L)) {  // the tables have L entries: report, and read the label as unknown
+        if (m == 0) atomicOr(status, 32);
+        lab = -1;
+    }
     float v;
     if (lab == -1) v = u_energy;                       // densecrf3d.h:118-121
     else v = (m == lab) ? p_en[lab] : n_en[lab];      // :123-126
@@ -300,10 +304,10 @@ int launch_axpy_norm(Ctx *ctx, float *out, const float *tmp, const float *norm, 
 }
 
 int mf_unary_from_label(Ctx *ctx, float *unary, const short *label_dev, int NT, int L, float u_energy,
-                        const float *n_en_dev, const float *p_en_dev) {
+                        const float *n_en_dev, const float *p_en_dev, int *status) {
     if (NT == 0) return LCCRF_OK;
     { LCCRF_KERNEL(ctx, "k_unary_from_label"); k_unary_from_label<<<cdiv((long long)NT * L, kThreads), kThreads, 0, ctx->stream>>>(unary, label_dev, NT, L, u_energy,
-                                                                                       n_en_dev, p_en_dev); }
+                                                                                       n_en_dev, p_en_dev, status); }
     LCCRF_CUDA(cudaGetLastError());
     return LCCRF_OK;
 }
