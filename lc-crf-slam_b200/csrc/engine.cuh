@@ -90,7 +90,9 @@ struct Ctx {
     cudaStream_t copy_stream = nullptr;  // uploads of the pipelined submit path (created on first use)
     cudaStream_t d2h_stream = nullptr;   // results of the pipelined submit path on their way to the host
     uint64_t launches = 0;
-    uint64_t scratch_gen = 0;  // bumped whenever a scratch buffer moves (captured graphs hold raw pointers)
+    // bumped whenever every captured graph goes stale: a scratch buffer moved (graphs hold raw pointers) or an option
+    // changed the launch sequence (lccrf_ctx_set_option)
+    uint64_t scratch_gen = 0;
     int opt_graphs = 1;
     int opt_fused = 1;
     // 1: splat sums every vertex row in point order (bit-identical to the reference's sequential loop);
@@ -144,10 +146,12 @@ int batch_init(Ctx *ctx, Batch &b, int B, const int *prob_ptr, int L, bool with_
 void batch_release(Ctx *ctx, Batch &b);
 // device status word: read (synchronises), clear, and turn the first error it holds into a return code
 int check_status(Ctx *ctx);
+int decode_status(int st);  // a status word -> error code (0: LCCRF_OK)
 
 // CUDA-graph replay of a launch sequence whose shape repeats.  The first run of a shape launches plainly; the second
-// runs once more uncaptured (every scratch buffer reaches its final size) and captures; later runs replay.  A caller
-// whose launch arguments change calls graph_drop, which makes the next run the first of a new shape.
+// runs once more uncaptured (every scratch buffer reaches its final size) and captures; later runs replay.  An object
+// keeps the key of every launch argument that can change between its runs (RunShape, FrameLaunch) its graph was captured
+// for and calls graph_drop when the next run's key differs, which makes that run the first of a new shape.
 struct GraphReplay {
     cudaGraphExec_t exec = nullptr;
     int same_shape_runs = 0;  // runs since the launch sequence last changed shape (a graph is captured on the 2nd)
@@ -271,7 +275,6 @@ struct DevMap {
     long long tail_seen = 0;      // last snapshot of the pool tail
     long long tail_unseen = 0;    // entries bulk loads added behind that snapshot (known exactly on the host)
     int epoch = 0;
-    uint64_t gen = 0;             // bumped whenever a device array moves (captured graphs hold raw pointers)
 };
 
 // a lccrf_map_delta whose arrays are in device memory
@@ -292,6 +295,13 @@ struct DeltaDev {
     const int *add_pt = nullptr, *add_kf = nullptr, *add_fid = nullptr;
     std::vector<int> erase_seg, add_seg;  // host copies of the segment boundaries (empty = one segment)
 };
+// bytes of the staged arrays of a delta (every array 256-byte aligned); with_keypoints = false when the new keyframes'
+// keypoints are copied straight from the host array
+size_t delta_stage_bytes(const lccrf_map_delta &d, int kp_stride, bool with_keypoints);
+// copy the delta's host arrays to `base` on stream st and describe them in `out`
+int delta_stage(const lccrf_map_delta &d, int kp_stride, bool with_keypoints, char *base, cudaStream_t st, DeltaDev *out);
+// explicit point ids name points the caller creates densely: raise the capacity to the largest id of the delta
+int delta_grow_points(DevMap *m, const lccrf_map_delta &d);
 
 int map_create(Ctx *ctx, int kp_stride, DevMap **out);
 void map_destroy(DevMap *m);
@@ -309,11 +319,14 @@ int map_begin_main_access(DevMap *m);   // context stream waits for the asynchro
 int map_end_main_access(DevMap *m);     // ... and marks the end of its access (external record node while capturing)
 int map_begin_async_mut(DevMap *m);     // map stream waits for the context stream's last access
 int map_end_async_mut(DevMap *m);
-// scope in which ctx->stream IS the map's stream: map.cu's launches, copies and allocations go there
+// scope in which ctx->stream IS the map's stream: map.cu's launches, copies and allocations go there (no-op when
+// enable is false)
 struct MapStreamScope {
     Ctx *c;
     cudaStream_t saved;
-    explicit MapStreamScope(DevMap *m) : c(m->ctx), saved(m->ctx->stream) { c->stream = m->mstream; }
+    explicit MapStreamScope(DevMap *m, bool enable = true) : c(m->ctx), saved(m->ctx->stream) {
+        if (enable) c->stream = m->mstream;
+    }
     ~MapStreamScope() { c->stream = saved; }
 };
 int map_reserve_pool(DevMap *m, long long entries);
@@ -402,7 +415,11 @@ int bf_match(Ctx *ctx, int B, int NQ, int max_nq, int max_nt, const int *q_ptr, 
 
 }  // namespace lccrf
 
-// opaque handle of include/lccrf.h (its entry points are spread over api.cu and images.cu)
+// opaque handles of include/lccrf.h (their entry points are spread over api.cu, frames.cu and images.cu)
 struct lccrf_ctx {
     lccrf::Ctx c;
+};
+
+struct lccrf_map {
+    lccrf::DevMap *m = nullptr;
 };

@@ -306,7 +306,6 @@ int reserve_keyframes(DevMap *m, int n) {
     LCCRF_TRY(grow_array(ctx, m->kf_packed, (size_t)m->kf_cap, (size_t)cap, true));
     LCCRF_TRY(grow_array(ctx, m->kp_tab, (size_t)m->kf_cap * m->kp_stride * 2, (size_t)cap * m->kp_stride * 2, true));
     m->kf_cap = (int)cap;
-    m->gen++;
     return map_publish(m);
 }
 
@@ -425,7 +424,6 @@ int map_reserve_points(DevMap *m, int n) {
     LCCRF_TRY(grow_array(ctx, m->pt_room, (size_t)m->pt_cap, (size_t)cap, true));
     LCCRF_TRY(grow_array(ctx, m->pt_stamp, (size_t)m->pt_cap, (size_t)cap, true));
     m->pt_cap = (int)cap;
-    m->gen++;
     return map_publish(m);
 }
 
@@ -442,7 +440,6 @@ int map_reserve_pool(DevMap *m, long long entries) {
     m->pool_cap = cap;
     { LCCRF_KERNEL(ctx, "k_map_set_word"); k_map_set_word<<<1, 1, 0, ctx->stream>>>(m->d_ctr + kCtrCap, (int)cap); }
     LCCRF_CUDA(cudaGetLastError());
-    m->gen++;
     return map_publish(m);
 }
 
@@ -463,7 +460,6 @@ int map_prepare(DevMap *m, const lccrf_map_delta &h) {
                 m->cam_set = true;
             } else if (m->ucam && memcmp(m->cam8, c8, sizeof(c8)) != 0) {
                 m->ucam = false;
-                m->gen++;
             }
         }
         if (h.kf_first + h.kf_count > m->n_kf) m->n_kf = h.kf_first + h.kf_count;
@@ -499,6 +495,70 @@ int map_prepare(DevMap *m, const lccrf_map_delta &h) {
         const long long known = m->tail_seen + m->tail_unseen;
         const long long want = 2 * known + 8LL * h.n_add + (1 << 16);
         if (want > m->pool_cap) LCCRF_TRY(map_reserve_pool(m, want));
+    }
+    return LCCRF_OK;
+}
+
+size_t delta_stage_bytes(const lccrf_map_delta &d, int kp_stride, bool with_keypoints) {
+    auto al = [](size_t b) { return (b + 255) / 256 * 256; };
+    size_t n = 0;
+    n += al((size_t)d.kf_count * 48) + al((size_t)d.kf_count * 16) * 2;
+    if (with_keypoints && d.kf_keypoints) n += al((size_t)d.kf_count * kp_stride * 8);
+    n += al((size_t)d.n_pose * 4) + al((size_t)d.n_pose * 48);
+    n += al((size_t)d.n_xyz * 4) + al((size_t)d.n_xyz * 12);
+    n += al((size_t)d.n_erase * 4) * 2 + al((size_t)d.n_bad * 4) + al((size_t)d.n_add * 4) * 3;
+    return n + 256;
+}
+
+int delta_stage(const lccrf_map_delta &d, int kp_stride, bool with_keypoints, char *base, cudaStream_t st, DeltaDev *out) {
+    size_t off = 0;
+    cudaError_t err = cudaSuccess;
+    auto put = [&](const void *src, size_t bytes) -> const void * {
+        if (!src || bytes == 0) return nullptr;
+        char *dst = base + off;
+        off += (bytes + 255) / 256 * 256;
+        cudaError_t e = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st);
+        if (e != cudaSuccess) err = e;
+        return dst;
+    };
+    DeltaDev o;
+    o.kf_first = d.kf_first;
+    o.kf_count = d.kf_count;
+    o.kf_pose = (const float *)put(d.kf_pose, (size_t)d.kf_count * 48);
+    o.kf_intr = (const float *)put(d.kf_intr, (size_t)d.kf_count * 16);
+    o.kf_bounds = (const float *)put(d.kf_bounds, (size_t)d.kf_count * 16);
+    if (with_keypoints) o.kf_keypoints = (const float *)put(d.kf_keypoints, (size_t)d.kf_count * kp_stride * 8);
+    o.n_pose = d.n_pose;
+    o.pose_kf = (const int *)put(d.pose_kf, (size_t)d.n_pose * 4);
+    o.pose = (const float *)put(d.pose, (size_t)d.n_pose * 48);
+    o.n_xyz = d.n_xyz;
+    o.xyz_id = (const int *)put(d.xyz_id, (size_t)d.n_xyz * 4);
+    o.xyz = (const float *)put(d.xyz, (size_t)d.n_xyz * 12);
+    o.n_erase = d.n_erase;
+    o.erase_pt = (const int *)put(d.erase_pt, (size_t)d.n_erase * 4);
+    o.erase_kf = (const int *)put(d.erase_kf, (size_t)d.n_erase * 4);
+    o.n_bad = d.n_bad;
+    o.bad_pt = (const int *)put(d.bad_pt, (size_t)d.n_bad * 4);
+    o.n_add = d.n_add;
+    o.add_pt = (const int *)put(d.add_pt, (size_t)d.n_add * 4);
+    o.add_kf = (const int *)put(d.add_kf, (size_t)d.n_add * 4);
+    o.add_fid = (const int *)put(d.add_fid, (size_t)d.n_add * 4);
+    if (d.n_erase_seg > 0) o.erase_seg.assign(d.erase_seg_ptr, d.erase_seg_ptr + d.n_erase_seg + 1);
+    if (d.n_add_seg > 0) o.add_seg.assign(d.add_seg_ptr, d.add_seg_ptr + d.n_add_seg + 1);
+    if (err != cudaSuccess) return fail(LCCRF_ERR_CUDA, std::string("map delta upload: ") + cudaGetErrorString(err));
+    *out = o;
+    return LCCRF_OK;
+}
+
+int delta_grow_points(DevMap *m, const lccrf_map_delta &d) {
+    if (d.n_xyz > 0 && d.xyz_id) {
+        int mx = -1;
+        for (int i = 0; i < d.n_xyz; i++) {
+            if (d.xyz_id[i] < 0) return fail(LCCRF_ERR_ARG, "map delta: negative point id");
+            if (d.xyz_id[i] > mx) mx = d.xyz_id[i];
+        }
+        LCCRF_TRY(map_reserve_points(m, mx + 1));
+        if (mx + 1 > m->n_pt) m->n_pt = mx + 1;
     }
     return LCCRF_OK;
 }
