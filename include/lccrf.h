@@ -56,6 +56,9 @@ int lccrf_ctx_set_stream(lccrf_ctx *ctx, void *cuda_stream);
 int lccrf_ctx_sync(lccrf_ctx *ctx);
 /* number of liblccrf kernels launched on this context so far (bench.py "gpu_launches") */
 uint64_t lccrf_ctx_kernel_launches(const lccrf_ctx *ctx);
+/* diagnostic: synchronises and counts the slots of the context's lattice-build hash scratch that are not empty.  Every
+ * build empties the slots it used, so the count is 0 whenever no build is in flight. */
+int lccrf_ctx_build_scratch_in_use(lccrf_ctx *ctx, long long *slots);
 /* option knobs (default):
  *   "ordered_splat" (1)  1: every lattice vertex sums its contributions in point order -- marginals bit-identical to the
  *                        reference; 0: fixed-shape tree reduction, 3x faster splat, marginals within 1e-4 of the reference

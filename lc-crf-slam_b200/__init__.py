@@ -73,6 +73,7 @@ SYMBOLS = {
     "lccrf_ctx_set_stream": (C.c_int, [_vp, _vp]),
     "lccrf_ctx_sync": (C.c_int, [_vp]),
     "lccrf_ctx_kernel_launches": (C.c_uint64, [_vp]),
+    "lccrf_ctx_build_scratch_in_use": (C.c_int, [_vp, _vp]),
     "lccrf_ctx_set_option": (C.c_int, [_vp, C.c_char_p, C.c_int]),
     "lccrf_ctx_profile_report": (C.c_int, [_vp, C.c_char_p, C.c_int]),
     "lccrf_lattice_create": (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.POINTER(_vp)]),
@@ -250,6 +251,12 @@ class Context:
     @property
     def kernel_launches(self) -> int:
         return int(self.lib.lccrf_ctx_kernel_launches(self.h))
+
+    def build_scratch_in_use(self) -> int:
+        """slots of the lattice-build hash scratch that are not empty (0 between builds); synchronises"""
+        n = C.c_longlong(0)
+        self._check(self.lib.lccrf_ctx_build_scratch_in_use(self.h, C.byref(n)))
+        return n.value
 
     # ---- free functions ----
     def exp_and_normalize(self, x, scale: float, relax: float = 1.0, prev=None) -> np.ndarray:

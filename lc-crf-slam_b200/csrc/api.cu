@@ -301,7 +301,7 @@ void lccrf_ctx_destroy(lccrf_ctx *h) {
         scratch_release(c, bs.hash_first, false);
         scratch_release(c, bs.hash_id, false);
         scratch_release(c, bs.ent_slot, false);
-        scratch_release(c, bs.blk_cnt, false);
+        scratch_release(c, bs.ids_status, false);
     }
     scratch_release(c, c->misc, false);
     scratch_release(c, c->feat, false);
@@ -348,6 +348,11 @@ int lccrf_ctx_sync(lccrf_ctx *h) {
 }
 
 uint64_t lccrf_ctx_kernel_launches(const lccrf_ctx *h) { return h ? h->c.launches : 0; }
+
+int lccrf_ctx_build_scratch_in_use(lccrf_ctx *h, long long *slots) {
+    if (!h || !slots) return fail(LCCRF_ERR_ARG, "NULL argument");
+    return build_scratch_in_use(&h->c, slots);
+}
 
 int lccrf_ctx_set_option(lccrf_ctx *h, const char *name, int value) {
     if (!h || !name) return fail(LCCRF_ERR_ARG, "NULL argument");

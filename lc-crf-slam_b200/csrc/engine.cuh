@@ -115,7 +115,10 @@ struct Ctx {
         size_t bytes = 0;
     };
     struct BuildScratch {  // lattice-build workspace; one set per concurrent branch
-        Scratch hash_keys[3], hash_first, hash_id, ent_slot, blk_cnt;
+        Scratch hash_keys[3], hash_first, hash_id, ent_slot, ids_status;
+        // hash_keys / hash_first are empty between builds (every build empties the slots it used); true while a build
+        // that may have left slots in use is in progress or failed before its clear was enqueued
+        bool hash_dirty = false;
     };
     BuildScratch bs[2];
     Scratch misc, feat, pinned_in, pinned_out, dev_io;
@@ -343,6 +346,8 @@ int lattice_set_create(Ctx *ctx, const Batch &b, int d, float w, int Lmax, Latti
 void lattice_set_destroy(Ctx *ctx, LatticeSet *ls);
 int lattice_set_build(Ctx *ctx, const Batch &b, LatticeSet *ls, const float *feat_dev);
 int lattice_set_ensure_L(Ctx *ctx, LatticeSet *ls, int L);  // (re)allocate the filter workspace for L labels
+// synchronises; slots of both branches' hash scratch that are not empty (0 between builds)
+int build_scratch_in_use(Ctx *ctx, long long *slots);
 // vertex-sorted CSR of a built lattice set (csr.cu)
 int csr_create(Ctx *ctx, const Batch &b, LatticeSet *ls);
 void csr_destroy(Ctx *ctx, LatticeSet *ls);

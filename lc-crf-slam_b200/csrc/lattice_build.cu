@@ -4,13 +4,14 @@
 //   k_embed<d>    elevate / round / rank / barycentric / keys for every point (incl. the reference's
 //                 phantom lanes, :294-299) and atomicCAS insertion of each key into a per-problem
 //                 open-addressing region; atomicMin records the FIRST scan position of every vertex.
-//   k_mark / k_scan_blocks / k_assign / k_vbase
-//                 canonical ids: the reference's id of a vertex is the number of distinct keys whose
+//   k_vertex_ids  canonical ids: the reference's id of a vertex is the number of distinct keys whose
 //                 first occurrence precedes its own in the k-major / remainder-minor scan (:371-377,
 //                 HashTableCPU::find :146).  That is an exclusive prefix sum over "is first occurrence"
 //                 flags in scan order -- no sort needed, and ids are bit-identical to the reference.
+//                 One launch: a chained scan with decoupled look-back.
 //   k_offsets     offset_[point][remainder] = id
 //   k_neighbours<d>  blur_neighbors_ (:408-421) by hash lookups of key -/+ 1 (axis j: +/- d)
+//   k_hash_clear<d>  empties the slots the build used, so the hash regions need no clear before the next build
 //
 // All arithmetic of the embedding is IEEE fp32 with every operation individually rounded
 // (__fmul_rn/__fadd_rn/__fsub_rn, file compiled with -fmad=false): the reference is built without
@@ -38,7 +39,6 @@ struct BuildParams {
     int *first;            // [slots] first scan position of the vertex stored in a last-level slot
     int *tab_id;           // [slots] global vertex id of a last-level slot
     int *ent_slot;         // [(NT+B)*D] last-level slot per scan position, -1 for inactive phantom entries
-    int *blk_cnt;          // per-block first-occurrence counts / offsets
     float *bary;           // [NT*D]
     int *offset;           // [NT*D]
     int2 *nbr;             // [D][Vcap]
@@ -215,89 +215,114 @@ __device__ __forceinline__ bool is_first(const BuildParams &p, int s, int S, int
     return slot >= 0 && __ldg(p.first + slot) == s;
 }
 
-template <int D>
-__global__ void __launch_bounds__(kThreads) k_mark(BuildParams p) {
-    const int S = (p.NT + p.B) * D;
-    const int s = blockIdx.x * kThreads + threadIdx.x;
-    int slot;
-    int cnt = __syncthreads_count(is_first(p, s, S, slot));
-    if (threadIdx.x == 0) p.blk_cnt[blockIdx.x] = cnt;
+// Single-pass chained scan (decoupled look-back).  A tile of kIdTile scan positions counts its flags, publishes the
+// count, adds the counts / prefixes of the tiles in front and publishes its inclusive prefix.  Tiles are numbered by an
+// atomic ticket, so a tile only ever waits on tiles that are already running.  The status words and the ticket
+// (ids_status, cleared before every launch) hold {flag (1: count, 2: inclusive prefix), value}.
+constexpr int kIdThreads = 1024;
+constexpr int kIdItems = 4;
+constexpr int kIdTile = kIdThreads * kIdItems;
+constexpr unsigned long long kIdCount = 1ull << 32, kIdPrefix = 2ull << 32;
+
+__device__ __forceinline__ void id_publish(unsigned long long *p, unsigned long long w) {
+    asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(w) : "memory");
+}
+__device__ __forceinline__ unsigned long long id_poll(const unsigned long long *p) {
+    unsigned long long w;
+    asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(w) : "l"(p) : "memory");
+    return w;
 }
 
-__global__ void __launch_bounds__(1024) k_scan_blocks(int *blk, int nblk, int *total_out) {
-    __shared__ int warp_sums[32];
-    __shared__ int carry_s;
-    if (threadIdx.x == 0) carry_s = 0;
+// writes tab_id, vert_slot, vert_prob, vbase[0..B]
+template <int D>
+__global__ void __launch_bounds__(kIdThreads) k_vertex_ids(BuildParams p, unsigned long long *ids_status, int ntiles) {
+    __shared__ int s_excl[kIdItems * 32];       // per 32-position group (scan order): flags in front of it inside the tile
+    __shared__ unsigned s_bal[kIdItems * 32];   // per group: its flags
+    __shared__ int s_tile, s_prefix, s_total;
+    if (threadIdx.x == 0) s_tile = (int)atomicAdd(ids_status + ntiles, 1ull);
     __syncthreads();
+    const int tile = s_tile;
+    const int S = (p.NT + p.B) * D;
+    const int s0 = tile * kIdTile;
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    for (int start = 0; start < nblk; start += 1024) {
-        int idx = start + threadIdx.x;
-        int v = idx < nblk ? blk[idx] : 0;
-        int x = v;
+    int slot[kIdItems];
+    unsigned bal[kIdItems];
+#pragma unroll
+    for (int j = 0; j < kIdItems; j++) {
+        const bool f = is_first(p, s0 + j * kIdThreads + threadIdx.x, S, slot[j]);
+        bal[j] = __ballot_sync(0xffffffffu, f);
+        if (!f) slot[j] = -1;
+        if (lane == 0) s_bal[j * 32 + wid] = bal[j];
+    }
+    __syncthreads();
+    if (wid == 0) {
+        int c[kIdItems], sum = 0;
+#pragma unroll
+        for (int k = 0; k < kIdItems; k++) {
+            c[k] = __popc(s_bal[lane * kIdItems + k]);
+            sum += c[k];
+        }
+        int incl = sum;
 #pragma unroll
         for (int o = 1; o < 32; o <<= 1) {
-            int y = __shfl_up_sync(0xffffffffu, x, o);
-            if (lane >= o) x += y;
+            const int y = __shfl_up_sync(0xffffffffu, incl, o);
+            if (lane >= o) incl += y;
         }
-        if (lane == 31) warp_sums[wid] = x;
-        __syncthreads();
-        if (wid == 0) {
-            int ws = warp_sums[lane];
+        int run = incl - sum;
 #pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                int y = __shfl_up_sync(0xffffffffu, ws, o);
-                if (lane >= o) ws += y;
+        for (int k = 0; k < kIdItems; k++) {
+            s_excl[lane * kIdItems + k] = run;
+            run += c[k];
+        }
+        const int total = __shfl_sync(0xffffffffu, incl, 31);
+        int prefix = 0;
+        if (tile > 0) {
+            if (lane == 0) id_publish(ids_status + tile, kIdCount | (unsigned)total);
+            for (int pred = tile - 1;;) {
+                const int t = pred - lane;
+                const unsigned long long w = t >= 0 ? id_poll(ids_status + t) : kIdPrefix;
+                if (__any_sync(0xffffffffu, (w >> 32) == 0)) continue;  // a tile in the window has not published yet
+                const unsigned pm = __ballot_sync(0xffffffffu, (w >> 32) == 2);
+                const int stop = pm ? __ffs(pm) - 1 : 31;  // nearest inclusive prefix ends the walk
+                int v = lane <= stop ? (int)(unsigned)w : 0;
+#pragma unroll
+                for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+                prefix += v;
+                if (pm) break;
+                pred -= 32;
             }
-            warp_sums[lane] = ws;  // inclusive
         }
-        __syncthreads();
-        int carry = carry_s;
-        int excl = carry + (wid ? warp_sums[wid - 1] : 0) + (x - v);
-        if (idx < nblk) blk[idx] = excl;
-        __syncthreads();
-        if (threadIdx.x == 1023) carry_s = carry + warp_sums[31];
-        __syncthreads();
+        if (lane == 0) {
+            id_publish(ids_status + tile, kIdPrefix | (unsigned)(prefix + total));
+            s_prefix = prefix;
+            s_total = total;
+        }
     }
-    if (threadIdx.x == 0) *total_out = carry_s;
-}
-
-template <int D>
-__global__ void __launch_bounds__(kThreads) k_assign(BuildParams p) {
-    __shared__ int warp_cnt[kThreads / 32];
-    const int S = (p.NT + p.B) * D;
-    const int s = blockIdx.x * kThreads + threadIdx.x;
-    int slot;
-    const bool flag = is_first(p, s, S, slot);
-    const unsigned bal = __ballot_sync(0xffffffffu, flag);
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    if (lane == 0) warp_cnt[wid] = __popc(bal);
     __syncthreads();
-    if (flag) {
-        int id = __ldg(p.blk_cnt + blockIdx.x) + __popc(bal & ((1u << lane) - 1u));
-        for (int w = 0; w < wid; w++) id += warp_cnt[w];
-        p.tab_id[slot] = id;
-        p.vert_slot[id] = slot;
-        p.vert_prob[id] = pseudo_problem(p.prob_ptr, p.B, s / D);
-    }
-}
-
-// vbase[b] = number of first occurrences before problem b's first scan position; one warp per problem
-template <int D>
-__global__ void __launch_bounds__(kThreads) k_vbase(BuildParams p) {
-    const int b = (blockIdx.x * kThreads + threadIdx.x) >> 5;
-    const int lane = threadIdx.x & 31;
-    if (b >= p.B) return;
-    const int S = (p.NT + p.B) * D;
-    const int sb = (__ldg(p.prob_ptr + b) + b) * D;
-    const int blk = sb / kThreads;
-    int cnt = 0;
-    for (int s = blk * kThreads + lane; s < sb; s += 32) {
-        int slot;
-        cnt += is_first(p, s, S, slot) ? 1 : 0;
-    }
+    const int prefix = s_prefix;
 #pragma unroll
-    for (int o = 16; o; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-    if (lane == 0) p.vbase[b] = __ldg(p.blk_cnt + blk) + cnt;
+    for (int j = 0; j < kIdItems; j++) {
+        if (slot[j] >= 0) {
+            const int s = s0 + j * kIdThreads + threadIdx.x;
+            const int id = prefix + s_excl[j * 32 + wid] + __popc(bal[j] & ((1u << lane) - 1u));
+            p.tab_id[slot[j]] = id;
+            p.vert_slot[id] = slot[j];
+            p.vert_prob[id] = pseudo_problem(p.prob_ptr, p.B, s / D);
+        }
+    }
+    // vbase[b] = number of first occurrences in front of problem b's first scan position (the phantom point keeps
+    // every problem's first position inside [0, S), so exactly one tile writes it)
+    const int s1 = s0 + kIdTile;
+    const int b0 = s0 < S ? pseudo_problem(p.prob_ptr, p.B, s0 / D) : p.B;
+    for (int b = b0 + (int)threadIdx.x; b < p.B; b += kIdThreads) {
+        const int sb = (__ldg(p.prob_ptr + b) + b) * D;
+        if (sb >= s1) break;
+        if (sb >= s0) {
+            const int q = sb - s0, g = q >> 5;
+            p.vbase[b] = prefix + s_excl[g] + __popc(s_bal[g] & ((1u << (q & 31)) - 1u));
+        }
+    }
+    if (tile == ntiles - 1 && threadIdx.x == 0) p.vbase[p.B] = prefix + s_total;
 }
 
 template <int D>
@@ -365,22 +390,47 @@ __global__ void __launch_bounds__(kThreads) k_neighbours(BuildParams p) {
     }
 }
 
+// Return the slots this build used to the empty state (key 0, first 0x7f7f7f7f): the last-level slot of every vertex
+// and, for d >= 4, the slots of its key chain at the earlier levels.  Those are shared between vertices; atomicExch
+// lets exactly one of the threads that reach a slot read its link to the level below.
 template <int d>
-int launch_build(Ctx *ctx, const BuildParams &p) {
+__global__ void __launch_bounds__(kThreads) k_hash_clear(BuildParams p) {
+    constexpr int NLEV = num_levels(d);
+    const int V = __ldg(p.vbase + p.B);
+    for (int id = blockIdx.x * kThreads + threadIdx.x; id < V; id += gridDim.x * kThreads) {
+        int slot = __ldg(p.vert_slot + id);
+        p.first[slot] = 0x7f7f7f7f;
+        if (NLEV == 1) {
+            p.key[0][slot] = 0ull;
+            continue;
+        }
+        const int base = __ldg(p.tab_base + __ldg(p.vert_prob + id));
+        uint64_t w = p.key[NLEV - 1][slot];
+        p.key[NLEV - 1][slot] = 0ull;
+#pragma unroll
+        for (int lev = NLEV - 2; lev >= 0 && w != 0ull; lev--) {
+            slot = base + (int)((w >> 32) & 0x7fffffffu);
+            w = atomicExch((unsigned long long *)p.key[lev] + slot, 0ull);
+        }
+    }
+}
+
+template <int d>
+int launch_build(Ctx *ctx, const BuildParams &p, unsigned long long *ids_status) {
     constexpr int D = d + 1;
     cudaStream_t st = ctx->stream;
     const int NP = p.NT + p.B;
     const long long S = (long long)NP * D;
-    const int nblk = cdiv(S, kThreads);
+    const int ntiles = S > 0 ? cdiv(S, kIdTile) : 1;
+    const int vgrid = persistent_grid((long long)p.Vcap, kThreads, 4);
     { LCCRF_KERNEL(ctx, "k_embed"); k_embed<d><<<cdiv(NP, kThreads), kThreads, 0, st>>>(p); }
-    { LCCRF_KERNEL(ctx, "k_mark"); k_mark<D><<<nblk, kThreads, 0, st>>>(p); }
-    { LCCRF_KERNEL(ctx, "k_scan_blocks"); k_scan_blocks<<<1, 1024, 0, st>>>(p.blk_cnt, nblk, p.vbase + p.B); }
-    { LCCRF_KERNEL(ctx, "k_assign"); k_assign<D><<<nblk, kThreads, 0, st>>>(p); }
-    { LCCRF_KERNEL(ctx, "k_vbase"); k_vbase<D><<<cdiv((long long)p.B * 32, kThreads), kThreads, 0, st>>>(p); }
+    LCCRF_CUDA(cudaMemsetAsync(ids_status, 0, ((size_t)ntiles + 1) * sizeof(unsigned long long), st));
+    { LCCRF_KERNEL(ctx, "k_vertex_ids"); k_vertex_ids<D><<<ntiles, kIdThreads, 0, st>>>(p, ids_status, ntiles); }
     if (p.NT > 0) {
         { LCCRF_KERNEL(ctx, "k_offsets"); k_offsets<D><<<cdiv(p.NT, kThreads), kThreads, 0, st>>>(p); }
     }
-    { LCCRF_KERNEL(ctx, "k_neighbours"); k_neighbours<d><<<persistent_grid((long long)p.Vcap, kThreads, 4), kThreads, 0, st>>>(p); }
+    { LCCRF_KERNEL(ctx, "k_neighbours"); k_neighbours<d><<<vgrid, kThreads, 0, st>>>(p); }
+    { LCCRF_KERNEL(ctx, "k_hash_clear"); k_hash_clear<d><<<vgrid, kThreads, 0, st>>>(p); }
     LCCRF_CUDA(cudaGetLastError());
     return LCCRF_OK;
 }
@@ -504,22 +554,30 @@ void lattice_set_destroy(Ctx *ctx, LatticeSet *ls) {
     delete ls;
 }
 
-int lattice_set_build(Ctx *ctx, const Batch &b, LatticeSet *ls, const float *feat_dev) {
+namespace {
+
+// hash scratch, build kernels up to k_hash_clear
+int build_enqueue(Ctx *ctx, const Batch &b, LatticeSet *ls, const float *feat_dev, Ctx::BuildScratch &bs, bool dirty) {
     const int d = ls->d, D = ls->D;
     const long long slots = ls->tab_slots;
     const int NLEV = num_levels(d);
-    Ctx::BuildScratch &bs = ctx->bs[ctx->branch];
-    for (int lev = 0; lev < NLEV; lev++) {
-        LCCRF_TRY(ctx_scratch(ctx, bs.hash_keys[lev], (size_t)slots * sizeof(uint64_t)));
-        LCCRF_CUDA(cudaMemsetAsync(bs.hash_keys[lev].p, 0, (size_t)slots * sizeof(uint64_t), ctx->stream));
+    auto hash_region = [&](Ctx::Scratch &s, size_t bytes, int fill) -> int {
+        const size_t had = s.p ? s.bytes : 0;  // ctx_scratch changes the size whenever it allocates
+        LCCRF_TRY(ctx_scratch(ctx, s, bytes));
+        if (s.bytes != had || dirty) LCCRF_CUDA(cudaMemsetAsync(s.p, fill, s.bytes, ctx->stream));
+        return LCCRF_OK;
+    };
+    for (int lev = 0; lev < NLEV; lev++) LCCRF_TRY(hash_region(bs.hash_keys[lev], (size_t)slots * sizeof(uint64_t), 0));
+    LCCRF_TRY(hash_region(bs.hash_first, (size_t)slots * sizeof(int), 0x7f));
+    if (dirty) {  // levels this build does not use may hold keys of a deeper lattice's failed build
+        for (int lev = NLEV; lev < 3; lev++)
+            if (bs.hash_keys[lev].p) LCCRF_CUDA(cudaMemsetAsync(bs.hash_keys[lev].p, 0, bs.hash_keys[lev].bytes, ctx->stream));
     }
-    LCCRF_TRY(ctx_scratch(ctx, bs.hash_first, (size_t)slots * sizeof(int)));
-    LCCRF_CUDA(cudaMemsetAsync(bs.hash_first.p, 0x7f, (size_t)slots * sizeof(int), ctx->stream));
     LCCRF_TRY(ctx_scratch(ctx, bs.hash_id, (size_t)slots * sizeof(int)));
     const long long S = ((long long)b.NT + b.B) * D;
     LCCRF_TRY(ctx_scratch(ctx, bs.ent_slot, (size_t)S * sizeof(int)));
-    const int nblk = cdiv(S, kThreads);
-    LCCRF_TRY(ctx_scratch(ctx, bs.blk_cnt, (size_t)(nblk + 1) * sizeof(int)));
+    const long long ntiles = S > 0 ? cdiv(S, kIdTile) : 1;
+    LCCRF_TRY(ctx_scratch(ctx, bs.ids_status, (size_t)(ntiles + 1) * sizeof(unsigned long long)));
 
     BuildParams p;
     memset(&p, 0, sizeof(p));
@@ -532,7 +590,6 @@ int lattice_set_build(Ctx *ctx, const Batch &b, LatticeSet *ls, const float *fea
     p.first = (int *)bs.hash_first.p;
     p.tab_id = (int *)bs.hash_id.p;
     p.ent_slot = (int *)bs.ent_slot.p;
-    p.blk_cnt = (int *)bs.blk_cnt.p;
     p.bary = ls->bary;
     p.offset = ls->offset;
     p.nbr = ls->nbr;
@@ -546,18 +603,67 @@ int lattice_set_build(Ctx *ctx, const Batch &b, LatticeSet *ls, const float *fea
     for (int i = 0; i < d; i++) p.scale[i] = (float)(1.0 / sqrt((double)((i + 2) * (i + 1))) * (double)inv_std_dev);
     p.invD = 1.0f / (d + 1);
     p.fD = (float)(d + 1);
+    unsigned long long *ids_status = (unsigned long long *)bs.ids_status.p;
     int rc = LCCRF_ERR_ARG;
     switch (d) {
-        case 1: rc = launch_build<1>(ctx, p); break;
-        case 2: rc = launch_build<2>(ctx, p); break;
-        case 3: rc = launch_build<3>(ctx, p); break;
-        case 4: rc = launch_build<4>(ctx, p); break;
-        case 5: rc = launch_build<5>(ctx, p); break;
-        case 6: rc = launch_build<6>(ctx, p); break;
-        case 7: rc = launch_build<7>(ctx, p); break;
+        case 1: rc = launch_build<1>(ctx, p, ids_status); break;
+        case 2: rc = launch_build<2>(ctx, p, ids_status); break;
+        case 3: rc = launch_build<3>(ctx, p, ids_status); break;
+        case 4: rc = launch_build<4>(ctx, p, ids_status); break;
+        case 5: rc = launch_build<5>(ctx, p, ids_status); break;
+        case 6: rc = launch_build<6>(ctx, p, ids_status); break;
+        case 7: rc = launch_build<7>(ctx, p, ids_status); break;
         default: return fail(LCCRF_ERR_ARG, "unsupported feature dimension");
     }
-    LCCRF_TRY(rc);
+    return rc;
+}
+
+}  // namespace
+
+__global__ void k_hash_in_use(const uint64_t *key, const int *first, long long n, unsigned long long *count) {
+    unsigned long long c = 0;
+    for (long long i = (long long)blockIdx.x * kThreads + threadIdx.x; i < n; i += (long long)gridDim.x * kThreads)
+        c += (key && key[i] != 0ull) || (first && first[i] != 0x7f7f7f7f);
+    if (c) atomicAdd(count, c);
+}
+
+int build_scratch_in_use(Ctx *ctx, long long *slots) {
+    unsigned long long *d_count = nullptr, h_count = 0;
+    LCCRF_CUDA(cudaStreamSynchronize(ctx->stream));
+    if (ctx->aux_stream) LCCRF_CUDA(cudaStreamSynchronize(ctx->aux_stream));
+    LCCRF_CUDA(cudaMalloc(&d_count, sizeof(unsigned long long)));
+    cudaError_t e = cudaMemset(d_count, 0, sizeof(unsigned long long));
+    for (const Ctx::BuildScratch &bs : ctx->bs) {
+        for (const Ctx::Scratch &k : bs.hash_keys)
+            if (e == cudaSuccess && k.p) {
+                k_hash_in_use<<<persistent_grid((long long)(k.bytes / 8), kThreads, 4), kThreads>>>((const uint64_t *)k.p, nullptr, (long long)(k.bytes / 8), d_count);
+                e = cudaGetLastError();
+            }
+        if (e == cudaSuccess && bs.hash_first.p) {
+            k_hash_in_use<<<persistent_grid((long long)(bs.hash_first.bytes / 4), kThreads, 4), kThreads>>>(nullptr, (const int *)bs.hash_first.p, (long long)(bs.hash_first.bytes / 4), d_count);
+            e = cudaGetLastError();
+        }
+    }
+    if (e == cudaSuccess) e = cudaMemcpy(&h_count, d_count, sizeof(h_count), cudaMemcpyDeviceToHost);
+    cudaFree(d_count);
+    if (e != cudaSuccess) return fail(LCCRF_ERR_CUDA, std::string("build_scratch_in_use: ") + cudaGetErrorString(e));
+    *slots = (long long)h_count;
+    return LCCRF_OK;
+}
+
+int lattice_set_build(Ctx *ctx, const Batch &b, LatticeSet *ls, const float *feat_dev) {
+    Ctx::BuildScratch &bs = ctx->bs[ctx->branch];
+    // Between builds every hash region is empty (keys 0, first 0x7f7f7f7f): a build empties the slots it used
+    // (k_hash_clear), so only a freshly allocated buffer, or every buffer after a build that stopped before its clear,
+    // is cleared in full.  The scratch counts as dirty from here until k_hash_clear is enqueued.
+    const bool dirty = bs.hash_dirty;
+    bs.hash_dirty = true;
+    const int rc = build_enqueue(ctx, b, ls, feat_dev, bs, dirty);
+    if (rc != LCCRF_OK) {
+        ctx->scratch_gen++;  // captured graphs of other objects have no clear in front of their builds: drop them
+        return rc;
+    }
+    bs.hash_dirty = false;
     return csr_build(ctx, b, ls);
 }
 
