@@ -100,6 +100,10 @@ int lccrf_lattice_filter(lccrf_lattice *lat, float *out, const float *in, int L)
  * starts at +0 is unchanged by +-0 addends) and a cropped output. */
 int lccrf_lattice_filter_window(lccrf_lattice *lat, float *out, const float *in, int L, int in_offset, int out_offset,
                                 int in_size, int out_size);
+/* diagnostics of the ordered splat's long rows, the counters of lccrf_frames_debug_counters: out8 = {#long rows,
+ * #chunks, #pieces, compose tickets, chunk records applied in O(1), crossing windows applied, chunks summed for real,
+ * zero chunks} (the last four accumulate over the filter calls since the lattice was built) */
+int lccrf_lattice_debug_counters(const lccrf_lattice *lat, int *out8);
 
 /* ---------------------------------------------------------------- dense CRF -------------- */
 /* Replaces DenseCRF3D<M>(N) / DenseCRFCPU<M>(N)   densecrf3d.h:23-28, densecrf_cpu.h:22-27 */

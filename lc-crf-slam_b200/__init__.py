@@ -82,6 +82,7 @@ SYMBOLS = {
     "lccrf_lattice_export": (C.c_int, [_vp, _vp, _vp, _vp]),
     "lccrf_lattice_filter": (C.c_int, [_vp, _vp, _vp, C.c_int]),
     "lccrf_lattice_filter_window": (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
+    "lccrf_lattice_debug_counters": (C.c_int, [_vp, _vp]),
     "lccrf_crf_create": (C.c_int, [_vp, C.c_int, C.c_int, C.POINTER(_vp)]),
     "lccrf_crf_destroy": (None, [_vp]),
     "lccrf_crf_set_unary": (C.c_int, [_vp, _vp]),
@@ -150,6 +151,9 @@ SYMBOLS = {
     "lccrf_snapshot_frame_info": (C.c_int, [_vp, C.c_int, _vp]),
     "lccrf_snapshot_read_frame": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp]),
 }
+
+# names of the eight long-row splat counters (lccrf_lattice_debug_counters, lccrf_frames_debug_counters)
+_SCAN_COUNTERS = ("long_rows", "chunks", "pieces", "tickets", "rec_fast", "rec_cross", "rec_fallback", "rec_zero")
 
 _lib = None
 
@@ -357,6 +361,12 @@ class Lattice:
         out = np.empty((max(n_out, 0), L), dtype=np.float32)
         self.ctx._check(self.ctx.lib.lccrf_lattice_filter_window(self.h, _ptr(out), _ptr(x), L, in_offset, out_offset, in_size, out_size))
         return out
+
+    def debug_counters(self):
+        """long-row splat counters; rec_* accumulate over the filter calls since the lattice was built"""
+        out = np.zeros(8, dtype=np.int32)
+        self.ctx._check(self.ctx.lib.lccrf_lattice_debug_counters(self.h, _ptr(out)))
+        return dict(zip(_SCAN_COUNTERS, out.tolist()))
 
     def close(self):
         if getattr(self, "h", None):
@@ -717,7 +727,7 @@ class Frames:
     def debug_counters(self, k):
         out = np.zeros(8, dtype=np.int32)
         self.ctx._check(self.ctx.lib.lccrf_frames_debug_counters(self.h, k, _ptr(out)))
-        return dict(zip(("long_rows", "chunks", "pieces", "tickets", "rec_fast", "rec_cross", "rec_fallback", "rec_zero"), out.tolist()))
+        return dict(zip(_SCAN_COUNTERS, out.tolist()))
 
     def algorithmic_bytes(self):
         t, i, u = C.c_double(), C.c_double(), C.c_double()

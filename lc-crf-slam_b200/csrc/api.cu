@@ -520,6 +520,15 @@ int lccrf_lattice_filter(lccrf_lattice *lat, float *out, const float *in, int L)
     return lccrf_lattice_filter_window(lat, out, in, L, 0, 0, -1, -1);
 }
 
+int lccrf_lattice_debug_counters(const lccrf_lattice *lat, int *out8) {
+    if (!lat || !out8) return fail(LCCRF_ERR_ARG, "NULL argument");
+    Ctx *ctx = lat->ctx;
+    LCCRF_CUDA(cudaSetDevice(ctx->device));
+    LCCRF_CUDA(cudaMemcpyAsync(out8, lat->ls->row_counts, 8 * sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+    LCCRF_CUDA(cudaStreamSynchronize(ctx->stream));
+    return LCCRF_OK;
+}
+
 // ------------------------------------------------------------------ dense CRF
 int lccrf_crf_create(lccrf_ctx *h, int N, int L, lccrf_crf **out) {
     if (!h || !out) return fail(LCCRF_ERR_ARG, "NULL argument");

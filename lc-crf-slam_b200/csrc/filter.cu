@@ -47,6 +47,39 @@ __device__ __forceinline__ ScanPair scan_combine(ScanPair l, ScanPair r) {  // a
     return o;
 }
 
+// One product in ulps of the binade, q = c/u (a power-of-two scaling: exact unless it underflows, far below 1/2), split as n = floor(q) and its fraction
+// against 1/2: up = fraction > 1/2, tie = fraction == 1/2.  Read from floor(2q), which is exact; q - floor(q) is not
+// for -1/2 < q < 0, where q = -1/2 + 2^-25 would round to a fraction of exactly 1/2 and pass for a tie.
+// |q| >= 2^24, inf and NaN give n = +-2^24, which no safe range admits.  NONNEG: q >= 0 (a monotone chunk), where
+// q - floor(q) is exact and costs less.
+template <bool NONNEG = false>
+__device__ __forceinline__ void split_ulps(float q, int &n, bool &up, bool &tie) {
+    up = tie = false;
+    if (!(fabsf(q) < 16777216.0f)) {
+        n = q > 0.0f ? (1 << 24) : -(1 << 24);
+        return;
+    }
+    if (NONNEG) {
+        n = __float2int_rd(q);
+        const float fr = __fsub_rn(q, (float)n);
+        up = fr > 0.5f;
+        tie = fr == 0.5f;
+        return;
+    }
+    const float q2 = __fmul_rn(q, 2.0f);
+    const int i2 = __float2int_rd(q2);
+    n = i2 >> 1;
+    if (i2 & 1) {
+        tie = __int2float_rn(i2) == q2;
+        up = !tie;
+    }
+}
+
+// The increments are rounded on the grid of binade E, which is only the true grid while the exact running sum stays
+// in [2^E, 2^(E+1)).  Below 2^E the grid is twice as fine, so an exact sum in [2^E - u/2, 2^E - u/4) rounds to 2^E on
+// E's grid but not in fp32.  The lower bound of a safe range is therefore taken over the exact prefixes: an entry
+// contributes (its rounded prefix in front of it) + floor(q), below which the exact sum behind it cannot lie.
+
 template <int NW>
 struct ScanShared {
     ScanPair warp_tot[NW > 1 ? NW : 1];
@@ -154,29 +187,23 @@ __device__ float row_sum_exact(const int2 *__restrict__ ent, const float *__rest
 #pragma unroll
                 for (int k = 0; k < IT; k++) {
                     if (li0 + k >= st && li0 + k < n_chunk) {
-                        const float q = __fmul_rn(c[k], inv_u);
                         int ni;
-                        float fr = 0.0f;
-                        if (!(fabsf(q) < 16777216.0f)) {  // also NaN / inf: forces "leaves the binade"
-                            ni = q > 0.0f ? (1 << 24) : -(1 << 24);
-                        } else {
-                            ni = __float2int_rd(q);
-                            fr = __fsub_rn(q, (float)ni);  // exact, in [0, 1)
-                        }
-                        if (fr != 0.5f) {  // common case: the same increment for either parity
-                            const int inc1 = ni + (fr > 0.5f ? 1 : 0);
+                        bool up, tie;
+                        split_ulps(__fmul_rn(c[k], inv_u), ni, up, tie);
+                        lo0 = min(lo0, tot.a0 + ni);  // floor of the exact prefix behind this entry
+                        lo1 = min(lo1, tot.a1 + ni);
+                        if (!tie) {  // common case: the same increment for either parity
+                            const int inc1 = ni + (up ? 1 : 0);
                             tot.a0 += inc1;
                             tot.a1 += inc1;
-                        } else {           // tie: round half to even
+                        } else {     // tie: round half to even
                             ScanPair a;
                             a.a0 = ni + (ni & 1);
                             a.a1 = ni + ((ni + 1) & 1);
                             tot = scan_combine(tot, a);
                         }
                         hi0 = max(hi0, tot.a0);
-                        lo0 = min(lo0, tot.a0);
                         hi1 = max(hi1, tot.a1);
-                        lo1 = min(lo1, tot.a1);
                     }
                 }
             }
@@ -326,20 +353,18 @@ __device__ __forceinline__ void thread_composite(const float *c, int n_valid, fl
 #pragma unroll
     for (int q = 0; q < IT; q++) {
         if (q < n_valid) {
-            const float qv = __fmul_rn(c[q], inv_u);
             int ni;
-            float fr = 0.0f;
-            if (!(fabsf(qv) < 16777216.0f)) {  // also NaN / inf: forces "leaves the binade"
-                ni = qv > 0.0f ? (1 << 24) : -(1 << 24);
-            } else {
-                ni = __float2int_rd(qv);
-                fr = __fsub_rn(qv, (float)ni);  // exact, in [0, 1)
+            bool up, t;
+            split_ulps<MONO>(__fmul_rn(c[q], inv_u), ni, up, t);
+            if (!MONO) {  // floor of the exact prefix behind this entry
+                lo0 = min(lo0, tot.a0 + ni);
+                lo1 = min(lo1, tot.a1 + ni);
             }
-            if (fr != 0.5f) {  // common case: the same increment for either parity
-                const int inc1 = ni + (fr > 0.5f ? 1 : 0);
+            if (!t) {  // common case: the same increment for either parity
+                const int inc1 = ni + (up ? 1 : 0);
                 tot.a0 += inc1;
                 tot.a1 += inc1;
-            } else {           // tie: round half to even
+            } else {   // tie: round half to even
                 tie = true;
                 ScanPair a;
                 a.a0 = ni + (ni & 1);
@@ -348,9 +373,7 @@ __device__ __forceinline__ void thread_composite(const float *c, int n_valid, fl
             }
             if (!MONO) {
                 hi0 = max(hi0, tot.a0);
-                lo0 = min(lo0, tot.a0);
                 hi1 = max(hi1, tot.a1);
-                lo1 = min(lo1, tot.a1);
             }
         }
     }
