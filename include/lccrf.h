@@ -402,6 +402,19 @@ int lccrf_frames_set_visible(lccrf_frames *fr, lccrf_map *map, const lccrf_map_d
                              const float *kp2d, const int *kf_ptr);
 int lccrf_frames_submit_visible(lccrf_frames *fr, int slot, lccrf_map *map, const lccrf_map_delta *delta,
                                 const int *point_id, const float *kp2d, const int *kf_ptr, short *map_out, float *prob_out);
+/* Frame batch against several resident maps (several tracked sequences on one GPU): map m serves problems
+ * [map_prob[m], map_prob[m+1]) (map_prob [n_maps+1], first 0, last B, non-decreasing; a map may serve no problem and
+ * still carry a delta).  point_id [NT] names points of the problem's own map; kf_ptr (optional, [B+1]) slices in the
+ * problem's own map's keyframe indices: within a map's segment it starts at 0 and does not decrease, the segment's last
+ * problem ends at that map's keyframe count, and kf_ptr[B] is the keyframe count of the last problem's map.  deltas:
+ * NULL or [n_maps] (a zeroed delta = nothing to do), deltas[m] applied to maps[m] first.  Every map belongs to fr's
+ * context and appears once.  Per problem the results are bit-identical to lccrf_frames_set_visible on that problem's
+ * map.  Same lifetime rules as set_visible / submit_visible. */
+int lccrf_frames_set_visible_maps(lccrf_frames *fr, int n_maps, lccrf_map *const *maps, const lccrf_map_delta *deltas,
+                                  const int *map_prob, const int *point_id, const float *kp2d, const int *kf_ptr);
+int lccrf_frames_submit_visible_maps(lccrf_frames *fr, int slot, int n_maps, lccrf_map *const *maps,
+                                     const lccrf_map_delta *deltas, const int *map_prob, const int *point_id,
+                                     const float *kp2d, const int *kf_ptr, short *map_out, float *prob_out);
 /* Epipolar prior of the next run / submission of `slot` (RroughClassify's second branch, Tracking.cc:2001-2010):
  * p4 [NT] = mvFeatureMatchProb[fid] of every point (0.0 without a match, :2003); has_prior [B] (optional) = 0 for the
  * problems whose frame had no fundamental matrix (mvFeatureMatchProb.empty(), :1994) -- those take the first branch.

@@ -139,6 +139,8 @@ SYMBOLS = {
     "lccrf_map_export": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, _vp, C.c_longlong, _vp]),
     "lccrf_frames_set_visible": (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp]),
     "lccrf_frames_submit_visible": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "lccrf_frames_set_visible_maps": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "lccrf_frames_submit_visible_maps": (C.c_int, [_vp, C.c_int, C.c_int, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "lccrf_frames_set_prior": (C.c_int, [_vp, C.c_int, _vp, _vp]),
     "lccrf_frames_set_partition_outputs": (C.c_int, [_vp, C.c_int, _vp, _vp, _vp, _vp, _vp]),
     "lccrf_snapshot_writer_open": (C.c_int, [C.c_char_p, C.c_int, C.POINTER(_vp)]),
@@ -682,6 +684,40 @@ class Frames:
         self.ctx._check(self.ctx.lib.lccrf_frames_submit_visible(
             self.h, slot, mp.h, C.byref(delta) if delta is not None else None, _ptr(point_id), _ptr(kp2d), _ptr(kf_ptr),
             _ptr(map_out), _ptr(prob_out)))
+
+    def _maps_args(self, maps, map_prob, deltas):
+        """(handle array, delta array or None, map_prob int32) of a multi-map call; None entries of deltas are zeroed"""
+        hs = (_vp * len(maps))(*[mp.h for mp in maps])
+        mprob = _arr(map_prob, np.int32)
+        if mprob.size != len(maps) + 1:
+            raise LccrfError("map_prob must have one entry per map plus one")
+        ds = None
+        if deltas is not None:
+            if len(deltas) != len(maps):
+                raise LccrfError("deltas must have one entry per map")
+            ds = (MapDelta * len(maps))()
+            for i, d in enumerate(deltas):
+                if d is not None:
+                    C.memmove(C.byref(ds, i * C.sizeof(MapDelta)), C.byref(d), C.sizeof(MapDelta))
+        return hs, ds, mprob
+
+    def set_visible_maps(self, maps, map_prob, point_id, kp2d, deltas=None, kf_ptr=None):
+        """frame batch against several resident maps: maps[m] serves problems [map_prob[m], map_prob[m+1]) and
+        takes deltas[m] (a MapDelta or None) first; point_id names points of the problem's own map.  Follow with run()."""
+        hs, ds, mprob = self._maps_args(maps, map_prob, deltas)
+        ids, kp, kfp = _arr(point_id, np.int32), _arr(kp2d, np.float32), _arr(kf_ptr, np.int32)
+        self.ctx._check(self.ctx.lib.lccrf_frames_set_visible_maps(self.h, len(maps), hs, ds, _ptr(mprob), _ptr(ids), _ptr(kp),
+                                                                 _ptr(kfp)))
+
+    def submit_visible_maps(self, slot, maps, map_prob, point_id, kp2d, map_out, prob_out, deltas=None, kf_ptr=None):
+        """pipelined set_visible_maps through HOST buffers (as submit_visible: contiguous int32 / float32 arrays, kept
+        alive with the deltas until wait(slot))"""
+        assert point_id.dtype == np.int32 and kp2d.dtype == np.float32 and (kf_ptr is None or kf_ptr.dtype == np.int32)
+        hs, ds, mprob = self._maps_args(maps, map_prob, deltas)
+        self._vis_keep = getattr(self, "_vis_keep", {})
+        self._vis_keep[slot] = (point_id, kp2d, deltas, kf_ptr, hs, ds, mprob)
+        self.ctx._check(self.ctx.lib.lccrf_frames_submit_visible_maps(
+            self.h, slot, len(maps), hs, ds, _ptr(mprob), _ptr(point_id), _ptr(kp2d), _ptr(kf_ptr), _ptr(map_out), _ptr(prob_out)))
 
     def set_prior(self, slot, p4=None, has_prior=None):
         """epipolar prior p4 [NT] float64 (+ per-problem flags [B] uint8) of the next run / submission of `slot`"""

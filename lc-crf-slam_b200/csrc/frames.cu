@@ -20,6 +20,7 @@ enum class FrameSource {
     kSnapshot,         // a map snapshot with keyframe indices and keypoints (set_map_inputs / submit_map)
     kSnapshotIndexed,  // a map snapshot with {keyframe, feature index} pairs; keypoints from lccrf_frames::kp_tab
     kVisible,          // ids of a device-resident map's points (set_visible / submit_visible)
+    kVisibleMaps,      // ids of the points of several resident maps, one segment of problems per map (*_visible_maps)
 };
 
 // Everything frames_enqueue passes to a kernel that can differ between runs of one frames object.  A captured graph
@@ -37,10 +38,15 @@ struct FrameLaunch {
     int nKF = 0, obs_kf_bytes = 0;
     long long nnz = 0;     // no kernel takes it, but a change has always meant a new capture
     int kf_slice_max = 0;  // largest per-problem keyframe slice (0 = unknown)
-    int kf_bucket = 0;     // shared-memory keyframe slots of the visible unary
+    int kf_bucket = 0;     // shared-memory keyframe slots of the visible unary (several maps: the largest bucket)
     bool ucam = false;     // every keyframe has the same intrinsics / image bounds: cam8 (all zero otherwise)
     float cam8[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     DevMap *map = nullptr;
+    // several maps: the maps in segment order, the problem segments, the padded point count and the segment table
+    std::vector<DevMap *> maps;
+    std::vector<int> map_prob;
+    int np = 0, n_seg = 0;
+    const void *segs = nullptr;
     const float *kp_tab = nullptr;  // resident keypoint table (indexed source), read when the run starts
     int kp_stride = 0;
     const double *p4 = nullptr;  // epipolar prior, or null
@@ -51,7 +57,8 @@ struct FrameLaunch {
                kf_bounds == o.kf_bounds && obs_ptr == o.obs_ptr && vis == o.vis && obs_kf == o.obs_kf &&
                kf_packed == o.kf_packed && kf_ptr == o.kf_ptr && nKF == o.nKF && obs_kf_bytes == o.obs_kf_bytes &&
                nnz == o.nnz && kf_slice_max == o.kf_slice_max && kf_bucket == o.kf_bucket && ucam == o.ucam &&
-               memcmp(cam8, o.cam8, sizeof(cam8)) == 0 && map == o.map && kp_tab == o.kp_tab &&
+               memcmp(cam8, o.cam8, sizeof(cam8)) == 0 && map == o.map && maps == o.maps && map_prob == o.map_prob &&
+               np == o.np && n_seg == o.n_seg && segs == o.segs && kp_tab == o.kp_tab &&
                kp_stride == o.kp_stride && p4 == o.p4 && p4_has == o.p4_has;
     }
 };
@@ -97,6 +104,13 @@ struct FrameInputs {
     size_t stage_cap = 0;
     DeltaDev delta;
     bool has_delta = false;
+    // several maps: the segment table (UnarySeg rows, unary.cu) and each problem's {first, end} keyframe slice ([2B]),
+    // and the staged deltas still to apply on their maps' streams (one per map that has one)
+    void *seg_tab = nullptr;
+    size_t seg_tab_cap = 0;
+    int *kf_pair = nullptr;
+    std::vector<DevMap *> delta_maps;
+    std::vector<DeltaDev> deltas;
     // epipolar prior (lccrf_frames_set_prior): host arrays as registered, device copies
     const double *h_p4 = nullptr;
     const unsigned char *h_p4_has = nullptr;
@@ -354,6 +368,135 @@ static int frames_upload_visible(lccrf_frames *fr, FrameInputs &in, cudaStream_t
     return frames_upload_finish(fr, in, st, kp2d, k);
 }
 
+static bool delta_empty(const lccrf_map_delta &d) {
+    return d.kf_count == 0 && d.n_pose == 0 && d.n_xyz == 0 && d.n_erase == 0 && d.n_bad == 0 && d.n_add == 0;
+}
+
+// frame points of several resident maps into input set `in` on stream `st`: map m serves problems [map_prob[m],
+// map_prob[m+1]) and takes its delta (deltas[m], optional) first.  The unary runs over a padded point space in which
+// every non-empty segment starts at a multiple of 256 points (unary_map_points_visible_multi).
+static int frames_upload_visible_maps(lccrf_frames *fr, FrameInputs &in, cudaStream_t st, int n_maps, lccrf_map *const *maps,
+                                      const lccrf_map_delta *deltas, const int *map_prob, const int *point_id,
+                                      const float *kp2d, const int *kf_ptr) {
+    Ctx *ctx = fr->ctx;
+    const int NT = fr->b.NT, B = fr->b.B;
+    const std::vector<int> &pp = fr->b.h_prob_ptr;
+    if (n_maps < 1) return fail(LCCRF_ERR_ARG, "n_maps must be >= 1");
+    if (!maps || !map_prob) return fail(LCCRF_ERR_ARG, "NULL argument");
+    if (NT > 0 && (!point_id || !kp2d)) return fail(LCCRF_ERR_ARG, "NULL argument");
+    std::vector<DevMap *> ms((size_t)n_maps);
+    for (int m = 0; m < n_maps; m++) {
+        if (!maps[m] || !maps[m]->m) return fail(LCCRF_ERR_ARG, "map is NULL");
+        ms[m] = maps[m]->m;
+        if (ms[m]->ctx != ctx) return fail(LCCRF_ERR_ARG, "map and frames belong to different contexts");
+        for (int j = 0; j < m; j++)
+            if (ms[j] == ms[m]) return fail(LCCRF_ERR_ARG, "a map appears twice in the map list");
+    }
+    if (map_prob[0] != 0 || map_prob[n_maps] != B) return fail(LCCRF_ERR_ARG, "map_prob must span [0, B]");
+    for (int m = 0; m < n_maps; m++)
+        if (map_prob[m + 1] < map_prob[m]) return fail(LCCRF_ERR_ARG, "map_prob must be non-decreasing");
+    const bool pipelined = st != ctx->stream;
+    auto has_delta = [&](int m) { return deltas && !delta_empty(deltas[m]); };
+    size_t need = 0;
+    for (int m = 0; m < n_maps; m++)
+        if (has_delta(m)) need += delta_stage_bytes(deltas[m], ms[m]->kp_stride, true);  // (a multiple of 256 bytes)
+    if (need > in.stage_cap) {
+        // rare (first steps): cudaFree waits for the device, so nothing still reads the old block
+        if (in.stage) LCCRF_CUDA(cudaFree(in.stage));
+        in.stage = nullptr;
+        in.stage_cap = 0;
+        const size_t cap = need + need / 2;
+        LCCRF_CUDA(cudaMalloc(&in.stage, cap));
+        in.stage_cap = cap;
+    }
+    for (int m = 0; m < n_maps; m++) {
+        if (!has_delta(m)) continue;
+        // as frames_upload_visible, per map: pipelined, the bookkeeping is stream-ordered on that map's stream
+        LCCRF_TRY(pipelined ? map_begin_async_mut(ms[m]) : map_begin_main_access(ms[m]));
+        MapStreamScope on_map_stream(ms[m], pipelined);
+        LCCRF_TRY(map_prepare(ms[m], deltas[m]));
+        LCCRF_TRY(delta_grow_points(ms[m], deltas[m]));
+    }
+    FrameLaunch k;
+    k.src = FrameSource::kVisibleMaps;
+    std::vector<int> pstart, cstart, count;
+    std::vector<MapHeader *> hdr;
+    std::vector<const float *> cams;
+    bool ucam = true;
+    for (int m = 0; m < n_maps; m++) {
+        const DevMap *d = ms[m];
+        k.kf_bucket = std::max(k.kf_bucket, (d->n_kf + 127) / 128 * 128);
+        const int c0 = pp[map_prob[m]], c1 = pp[map_prob[m + 1]];
+        if (c1 == c0) continue;
+        if (d->n_kf <= 0) return fail(LCCRF_ERR_STATE, "the map has no keyframes");
+        ucam = ucam && d->cam_set && d->ucam;
+        pstart.push_back(k.np);
+        cstart.push_back(c0);
+        count.push_back(c1 - c0);
+        hdr.push_back(d->d_hdr);
+        cams.push_back(d->cam8);
+        k.np += (c1 - c0 + 255) / 256 * 256;
+    }
+    pstart.push_back(k.np);
+    k.n_seg = (int)count.size();
+    k.ucam = k.n_seg > 0 && ucam;
+    // kf_ptr: within segment m, the slices of its problems in that map's keyframes -- they start at 0, do not decrease, and
+    // the segment's last problem ends at the map's keyframe count; kf_ptr[B] = that count for the last problem's map.
+    // The kernel reads a {first, end} pair per problem.
+    std::vector<int> pairs;
+    if (kf_ptr) {
+        pairs.resize((size_t)2 * B);
+        for (int m = 0; m < n_maps; m++) {
+            const int p0 = map_prob[m], p1 = map_prob[m + 1], n = ms[m]->n_kf;
+            if (p1 == p0) continue;
+            if (kf_ptr[p0] != 0) return fail(LCCRF_ERR_ARG, "kf_ptr must start every map's segment at 0");
+            for (int b = p0; b < p1; b++) {
+                const int lo = kf_ptr[b], hi = b + 1 == p1 ? n : kf_ptr[b + 1];
+                if (lo < 0 || hi < lo || hi > n) return fail(LCCRF_ERR_ARG, "kf_ptr out of range for the segment's map");
+                pairs[2 * b] = lo;
+                pairs[2 * b + 1] = hi;
+                k.kf_slice_max = std::max(k.kf_slice_max, hi - lo);
+            }
+            if (p1 == B && kf_ptr[B] != n) return fail(LCCRF_ERR_ARG, "kf_ptr[B] must be the last map's number of keyframes");
+        }
+    }
+    if (!in.vis) LCCRF_TRY(slot_alloc(ctx, in, st, in.vis, (size_t)(NT ? NT : 1) * 4));
+    if (kf_ptr && !in.kf_pair) LCCRF_TRY(slot_alloc(ctx, in, st, in.kf_pair, (size_t)2 * B * 4));
+    const size_t tb = unary_seg_table_bytes(k.n_seg);
+    if (tb > in.seg_tab_cap) {  // (a new table pointer: the slot's next run sees a new launch key)
+        LCCRF_TRY(slot_alloc(ctx, in, st, in.seg_tab, tb));
+        in.seg_tab_cap = tb;
+    }
+    std::vector<char> tab(tb);
+    unary_seg_table(k.n_seg, pstart.data(), cstart.data(), count.data(), hdr.data(), cams.data(), tab.data());
+    k.vis = in.vis;
+    k.kf_ptr = kf_ptr ? in.kf_pair : nullptr;
+    k.maps = ms;
+    k.map_prob.assign(map_prob, map_prob + n_maps + 1);
+    k.segs = in.seg_tab;
+    // every delta at its own 256-byte aligned offset of the slot's stage buffer
+    in.delta_maps.clear();
+    in.deltas.clear();
+    size_t off = 0;
+    for (int m = 0; m < n_maps; m++) {
+        if (!has_delta(m)) continue;
+        char *base = (char *)in.stage + off;
+        off += delta_stage_bytes(deltas[m], ms[m]->kp_stride, true);
+        DeltaDev dd;
+        LCCRF_TRY(delta_stage(deltas[m], ms[m]->kp_stride, pipelined, base, st, &dd));
+        if (pipelined) {  // applied on the map's stream once the upload has landed (frames_run_slot)
+            in.delta_maps.push_back(ms[m]);
+            in.deltas.push_back(dd);
+        } else {
+            LCCRF_TRY(map_apply_dev(ms[m], dd, deltas[m].kf_count > 0 ? deltas[m].kf_keypoints : nullptr));
+        }
+    }
+    LCCRF_CUDA(cudaMemcpyAsync(in.seg_tab, tab.data(), tb, cudaMemcpyHostToDevice, st));
+    if (kf_ptr && B) LCCRF_CUDA(cudaMemcpyAsync(in.kf_pair, pairs.data(), pairs.size() * 4, cudaMemcpyHostToDevice, st));
+    if (NT > 0) LCCRF_CUDA(cudaMemcpyAsync(in.vis, point_id, (size_t)NT * 4, cudaMemcpyHostToDevice, st));
+    return frames_upload_finish(fr, in, st, kp2d, k);
+}
+
 static int frames_enqueue(lccrf_frames *fr, const FrameLaunch &k) {
     Ctx *ctx = fr->ctx;
     Batch &b = fr->b;
@@ -374,6 +517,10 @@ static int frames_enqueue(lccrf_frames *fr, const FrameLaunch &k) {
         LCCRF_TRY(unary_map_points_visible(ctx, NT, k.vis, k.map->d_hdr, k.kf_bucket, fr->observs, fr->error, fr->depth,
                                            b.prob_ptr, k.kf_ptr, b.B, k.kf_slice_max, cam8));
         LCCRF_TRY(map_end_main_access(k.map));  // the map may change from here on (the next step's delta, on the map's stream)
+    } else if (k.src == FrameSource::kVisibleMaps) {
+        LCCRF_TRY(unary_map_points_visible_multi(ctx, k.np, k.n_seg, k.segs, k.vis, k.kf_bucket, fr->observs, fr->error,
+                                                 fr->depth, b.prob_ptr, k.kf_ptr, b.B, k.kf_slice_max, k.ucam));
+        for (DevMap *m : k.maps) LCCRF_TRY(map_end_main_access(m));
     } else if (k.src != FrameSource::kDirect) {
         LCCRF_TRY(unary_pack_kf(ctx, k.kf_packed, k.kf_pose, k.kf_intr, k.kf_bounds, k.nKF));
         LCCRF_TRY(unary_map_points_packed(ctx, NT, k.nKF, k.xyz, k.obs_ptr, k.obs_kf, k.obs_kf_bytes, k.obs_uv, k.kf_packed,
@@ -428,7 +575,21 @@ static int frames_run_slot(lccrf_frames *fr, FrameInputs &in, cudaStream_t uploa
         }
         LCCRF_TRY(map_end_async_mut(k.map));
     }
+    // several maps: each map's delta on that map's stream; the run waits for all of them
+    for (size_t i = 0; i < in.deltas.size(); i++) {
+        DevMap *m = in.delta_maps[i];
+        LCCRF_CUDA(cudaStreamWaitEvent(m->mstream, in.up_done, 0));
+        {
+            MapStreamScope on_map_stream(m);
+            LCCRF_TRY(map_apply_dev(m, in.deltas[i], nullptr));
+        }
+        LCCRF_TRY(map_end_async_mut(m));
+    }
+    in.deltas.clear();
+    in.delta_maps.clear();
     if (k.src == FrameSource::kVisible) LCCRF_TRY(map_begin_main_access(k.map));
+    if (k.src == FrameSource::kVisibleMaps)
+        for (DevMap *m : k.maps) LCCRF_TRY(map_begin_main_access(m));
     LCCRF_TRY(graph_run(ctx, in.graph, [&] { return frames_enqueue(fr, k); }));
     fr->ran = true;
     return LCCRF_OK;
@@ -534,6 +695,8 @@ static void frame_inputs_release(Ctx *ctx, FrameInputs &in) {
     dev_free(ctx, in.kf_packed);
     dev_free(ctx, in.kf_ptr);
     dev_free(ctx, in.vis);
+    dev_free(ctx, in.seg_tab);
+    dev_free(ctx, in.kf_pair);
     dev_free(ctx, in.out_stage);
     if (in.res_ready) cudaEventDestroy(in.res_ready);
     dev_free(ctx, in.p4);
@@ -645,6 +808,17 @@ int lccrf_frames_set_visible(lccrf_frames *fr, lccrf_map *map, const lccrf_map_d
     return LCCRF_OK;
 }
 
+int lccrf_frames_set_visible_maps(lccrf_frames *fr, int n_maps, lccrf_map *const *maps, const lccrf_map_delta *deltas,
+                                  const int *map_prob, const int *point_id, const float *kp2d, const int *kf_ptr) {
+    if (!fr) return fail(LCCRF_ERR_ARG, "frames is NULL");
+    LCCRF_CUDA(cudaSetDevice(fr->ctx->device));
+    LCCRF_TRY(frames_check_idle(fr));
+    LCCRF_TRY(frames_upload_visible_maps(fr, fr->in[0], fr->ctx->stream, n_maps, maps, deltas, map_prob, point_id, kp2d, kf_ptr));
+    // the host arrays (deltas included) are free on return
+    LCCRF_CUDA(cudaStreamSynchronize(fr->ctx->stream));
+    return LCCRF_OK;
+}
+
 int lccrf_frames_set_prior(lccrf_frames *fr, int slot, const double *p4, const unsigned char *has_prior) {
     if (!fr) return fail(LCCRF_ERR_ARG, "frames is NULL");
     if (slot < 0 || slot > 1) return fail(LCCRF_ERR_ARG, "slot must be 0 or 1");
@@ -744,6 +918,20 @@ int lccrf_frames_submit_visible(lccrf_frames *fr, int slot, lccrf_map *map, cons
     LCCRF_TRY(frames_submit_prologue(fr, slot, &in));
     tm.mark("prologue");
     LCCRF_TRY(frames_upload_visible(fr, *in, fr->ctx->copy_stream, map, delta, point_id, kp2d, kf_ptr));
+    tm.mark("upload");
+    const int rc = frames_submit_epilogue(fr, slot, *in, map_out, prob_out);
+    tm.mark("apply+run+results");
+    return rc;
+}
+
+int lccrf_frames_submit_visible_maps(lccrf_frames *fr, int slot, int n_maps, lccrf_map *const *maps,
+                                     const lccrf_map_delta *deltas, const int *map_prob, const int *point_id,
+                                     const float *kp2d, const int *kf_ptr, short *map_out, float *prob_out) {
+    FrameInputs *in = nullptr;
+    PhaseTimer tm(fr && fr->ctx->opt_trace);
+    LCCRF_TRY(frames_submit_prologue(fr, slot, &in));
+    tm.mark("prologue");
+    LCCRF_TRY(frames_upload_visible_maps(fr, *in, fr->ctx->copy_stream, n_maps, maps, deltas, map_prob, point_id, kp2d, kf_ptr));
     tm.mark("upload");
     const int rc = frames_submit_epilogue(fr, slot, *in, map_out, prob_out);
     tm.mark("apply+run+results");
@@ -867,14 +1055,24 @@ int lccrf_frames_algorithmic_bytes(lccrf_frames *fr, double *total, double *per_
     const FrameLaunch &k = fr->in[fr->last_slot].launch;
     long long nnz = k.nnz;
     int nKF = k.nKF;
-    if (k.src == FrameSource::kVisible) {  // observations of the visible points: counted on the device
-        nKF = k.map->n_kf;
+    if (k.src == FrameSource::kVisible || k.src == FrameSource::kVisibleMaps) {  // observations of the visible points: counted on the device
+        // (map, first point, end point) of every segment
+        std::vector<std::pair<DevMap *, std::pair<int, int>>> seg;
+        if (k.src == FrameSource::kVisible) seg.push_back({k.map, {0, fr->b.NT}});
+        for (size_t m = 0; m < k.maps.size(); m++)
+            seg.push_back({k.maps[m], {fr->b.h_prob_ptr[k.map_prob[m]], fr->b.h_prob_ptr[k.map_prob[m + 1]]}});
+        nKF = 0;
+        for (auto &g : seg) nKF += g.first->n_kf;
         nnz = 0;
         if (fr->b.NT > 0) {
             Ctx *ctx = fr->ctx;
             int *d_cnt = nullptr;
             LCCRF_TRY(dev_alloc(ctx, (void **)&d_cnt, (size_t)fr->b.NT * 4));
-            int rc = map_export_dev(k.map, fr->b.NT, k.vis, d_cnt);
+            int rc = LCCRF_OK;
+            for (auto &g : seg) {
+                const int c0 = g.second.first, c1 = g.second.second;
+                if (rc == LCCRF_OK && c1 > c0) rc = map_export_dev(g.first, c1 - c0, k.vis + c0, d_cnt + c0);
+            }
             std::vector<int> cnt((size_t)fr->b.NT);
             if (rc == LCCRF_OK) {
                 cudaError_t e = cudaMemcpyAsync(cnt.data(), d_cnt, cnt.size() * 4, cudaMemcpyDeviceToHost, ctx->stream);
