@@ -397,7 +397,8 @@ int lccrf_map_export(lccrf_map *map, int n, const int *point_id, int *obs_ptr, i
  * :1858), kp2d [NT*2] their keypoints in the frame.  `delta` (optional) is applied first.  kf_ptr as in
  * lccrf_frames_set_map_inputs.  set_visible uploads on the context's stream (follow with lccrf_frames_run);
  * submit_visible is the pipelined form (slot 0 / 1, uploads on the copy stream, results into map_out / prob_out, finish
- * with lccrf_frames_wait): host arrays, including the delta's, must stay valid until that wait returns. */
+ * with lccrf_frames_wait): host arrays, including the delta's, must stay valid until that wait returns.  Both equal
+ * lccrf_frames_set_visible_maps / submit_visible_maps with the one map {map}, map_prob {0, B} and deltas = delta. */
 int lccrf_frames_set_visible(lccrf_frames *fr, lccrf_map *map, const lccrf_map_delta *delta, const int *point_id,
                              const float *kp2d, const int *kf_ptr);
 int lccrf_frames_submit_visible(lccrf_frames *fr, int slot, lccrf_map *map, const lccrf_map_delta *delta,

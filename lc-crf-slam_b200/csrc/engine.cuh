@@ -388,20 +388,19 @@ int unary_map_points_packed(Ctx *ctx, int N, int nKF, const float *xyz, const in
                             int obs_kf_bytes, const float *obs_uv, const void *kf_packed, float *observs, float *error, float *depth,
                             const int *prob_ptr, const int *kf_ptr, int B, int kf_slice_max, const float *cam8,
                             const float *kp_tab, int kp_stride);
-int unary_map_points_visible(Ctx *ctx, int N, const int *vis, const MapHeader *map_hdr, int n_kf_bucket, float *observs,
-                             float *error, float *depth, const int *prob_ptr, const int *kf_ptr, int B, int kf_slice_max,
-                             const float *cam8);
-// Frame points of several resident maps in one launch (lccrf_frames_set_visible_maps): segment s = points
-// [cstart[s], cstart[s] + count[s]) of the batch, all from the map behind hdr[s], placed at padded start pstart[s] (a multiple
-// of 256; pstart[n_seg] = NP, the padded total).  unary_seg_table writes the table (unary_seg_table_bytes) into host memory
-// `out` for upload; cam8[s]: the map's camera when ucam.  kf_pair (optional, [2B]): {first, end} of each problem's keyframe
-// slice in its own map.  n_kf_bucket: the largest bucket of the maps.
+// Frame points named by map point ids against device-resident maps (lccrf_frames_set_visible_maps).  One map
+// (map_hdr != nullptr): the batch's N points, all of that map; cam8 its camera when it has one.  Several maps: segment s =
+// points [cstart[s], cstart[s] + count[s]) of the batch, all from the map behind hdr[s], placed at padded start pstart[s]
+// (a multiple of 256; pstart[n_seg] = N, the padded total).  unary_seg_table writes the table (unary_seg_table_bytes)
+// into host memory `out` for upload; cam8[s]: the map's camera when every map has one (the launch then passes a
+// non-null cam8).  kf_pair (optional, [2B]): {first, end} of each problem's keyframe slice in its own map.
+// n_kf_bucket: the largest bucket of the maps.
 size_t unary_seg_table_bytes(int n_seg);
 void unary_seg_table(int n_seg, const int *pstart, const int *cstart, const int *count, MapHeader *const *hdr,
                      const float *const *cam8, void *out);
-int unary_map_points_visible_multi(Ctx *ctx, int NP, int n_seg, const void *seg_table, const int *vis, int n_kf_bucket,
-                                   float *observs, float *error, float *depth, const int *prob_ptr, const int *kf_pair,
-                                   int B, int kf_slice_max, bool ucam);
+int unary_map_points_visible(Ctx *ctx, int N, const int *vis, const MapHeader *map_hdr, int n_seg, const void *seg_table,
+                             int n_kf_bucket, float *observs, float *error, float *depth, const int *prob_ptr,
+                             const int *kf_pair, int B, int kf_slice_max, const float *cam8);
 // kp_tab != nullptr: indexed observations -- obs_kf holds {keyframe, feature index} pairs (uint16 pairs when
 // obs_kf_bytes == 2, int32 pairs when 4), obs_uv is unused and the observed keypoint is kp_tab[kf*kp_stride + fid]
 int unary_map_points(Ctx *ctx, int N, const float *xyz, const int *obs_ptr, const int *obs_kf,

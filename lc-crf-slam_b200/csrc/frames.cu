@@ -19,8 +19,8 @@ enum class FrameSource {
     kDirect,           // the Tracking.cc:1849-1870 vectors (lccrf_frames_set_inputs / submit)
     kSnapshot,         // a map snapshot with keyframe indices and keypoints (set_map_inputs / submit_map)
     kSnapshotIndexed,  // a map snapshot with {keyframe, feature index} pairs; keypoints from lccrf_frames::kp_tab
-    kVisible,          // ids of a device-resident map's points (set_visible / submit_visible)
-    kVisibleMaps,      // ids of the points of several resident maps, one segment of problems per map (*_visible_maps)
+    kVisibleMaps,      // ids of the points of resident maps, one segment of problems per map (*_visible_maps;
+                       // set_visible / submit_visible pass a list of one map)
 };
 
 // Everything frames_enqueue passes to a kernel that can differ between runs of one frames object.  A captured graph
@@ -34,15 +34,16 @@ struct FrameLaunch {
     const int *obs_ptr = nullptr, *vis = nullptr;
     const void *obs_kf = nullptr;
     void *kf_packed = nullptr;
-    const int *kf_ptr = nullptr;  // [B+1] keyframe slice of each problem, or null
+    const int *kf_ptr = nullptr;  // keyframe slice of each problem ([B+1]; resident maps: {first, end} pairs), or null
     int nKF = 0, obs_kf_bytes = 0;
     long long nnz = 0;     // no kernel takes it, but a change has always meant a new capture
     int kf_slice_max = 0;  // largest per-problem keyframe slice (0 = unknown)
-    int kf_bucket = 0;     // shared-memory keyframe slots of the visible unary (several maps: the largest bucket)
-    bool ucam = false;     // every keyframe has the same intrinsics / image bounds: cam8 (all zero otherwise)
+    int kf_bucket = 0;     // shared-memory keyframe slots of the visible unary (the largest bucket of the maps)
+    bool ucam = false;     // every keyframe has the same intrinsics / image bounds: cam8 (all zero otherwise, and with
+                           // several maps, whose cameras travel in the segment table)
     float cam8[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-    DevMap *map = nullptr;
-    // several maps: the maps in segment order, the problem segments, the padded point count and the segment table
+    // resident maps: the maps in list order and the problem segments; several maps: the padded point count and the
+    // segment table
     std::vector<DevMap *> maps;
     std::vector<int> map_prob;
     int np = 0, n_seg = 0;
@@ -57,7 +58,7 @@ struct FrameLaunch {
                kf_bounds == o.kf_bounds && obs_ptr == o.obs_ptr && vis == o.vis && obs_kf == o.obs_kf &&
                kf_packed == o.kf_packed && kf_ptr == o.kf_ptr && nKF == o.nKF && obs_kf_bytes == o.obs_kf_bytes &&
                nnz == o.nnz && kf_slice_max == o.kf_slice_max && kf_bucket == o.kf_bucket && ucam == o.ucam &&
-               memcmp(cam8, o.cam8, sizeof(cam8)) == 0 && map == o.map && maps == o.maps && map_prob == o.map_prob &&
+               memcmp(cam8, o.cam8, sizeof(cam8)) == 0 && maps == o.maps && map_prob == o.map_prob &&
                np == o.np && n_seg == o.n_seg && segs == o.segs && kp_tab == o.kp_tab &&
                kp_stride == o.kp_stride && p4 == o.p4 && p4_has == o.p4_has;
     }
@@ -100,15 +101,13 @@ struct FrameInputs {
     int *vis = nullptr;      // [NT] map point ids
     void *out_stage = nullptr;     // per-slot copy of the results (marginals, labels, status word) on their way to the host
     cudaEvent_t res_ready = nullptr;
-    void *stage = nullptr;    // staged arrays of this step's map delta
+    void *stage = nullptr;    // staged arrays of this step's map deltas
     size_t stage_cap = 0;
-    DeltaDev delta;
-    bool has_delta = false;
-    // several maps: the segment table (UnarySeg rows, unary.cu) and each problem's {first, end} keyframe slice ([2B]),
-    // and the staged deltas still to apply on their maps' streams (one per map that has one)
-    void *seg_tab = nullptr;
-    size_t seg_tab_cap = 0;
-    int *kf_pair = nullptr;
+    // resident maps: the segment table (several maps; UnarySeg rows, unary.cu), then each problem's {first, end} keyframe
+    // slice ([2B]) -- written to the pinned h_tab and sent in one copy -- and the staged deltas still to apply on their
+    // maps' streams (one per map that has one)
+    void *tab = nullptr, *h_tab = nullptr;
+    size_t tab_cap = 0;
     std::vector<DevMap *> delta_maps;
     std::vector<DeltaDev> deltas;
     // epipolar prior (lccrf_frames_set_prior): host arrays as registered, device copies
@@ -312,69 +311,14 @@ static int frames_upload_map(lccrf_frames *fr, FrameInputs &in, cudaStream_t st,
     return frames_upload_finish(fr, in, st, kp2d, k);
 }
 
-// frame points named by ids of the resident map (+ the step's map delta) into input set `in` on stream `st`
-static int frames_upload_visible(lccrf_frames *fr, FrameInputs &in, cudaStream_t st, lccrf_map *map, const lccrf_map_delta *delta,
-                                 const int *point_id, const float *kp2d, const int *kf_ptr) {
-    Ctx *ctx = fr->ctx;
-    if (!map || !map->m) return fail(LCCRF_ERR_ARG, "map is NULL");
-    DevMap *m = map->m;
-    if (m->ctx != ctx) return fail(LCCRF_ERR_ARG, "map and frames belong to different contexts");
-    const int NT = fr->b.NT, B = fr->b.B;
-    if (NT > 0 && (!point_id || !kp2d)) return fail(LCCRF_ERR_ARG, "NULL argument");
-    const bool pipelined = st != ctx->stream;
-    if (delta) {
-        const size_t need = delta_stage_bytes(*delta, m->kp_stride, true);
-        if (need > in.stage_cap) {
-            // rare (first steps): cudaFree waits for the device, so nothing still reads the old block
-            if (in.stage) LCCRF_CUDA(cudaFree(in.stage));
-            in.stage = nullptr;
-            in.stage_cap = 0;
-            const size_t cap = need + need / 2;
-            LCCRF_CUDA(cudaMalloc(&in.stage, cap));
-            in.stage_cap = cap;
-        }
-        // host-side bookkeeping + capacity growth.  Pipelined: stream-ordered on the MAP's stream behind the last access
-        // of the context's stream (an array that moves is freed there, and the previous step's unary may still read it)
-        LCCRF_TRY(pipelined ? map_begin_async_mut(m) : map_begin_main_access(m));
-        MapStreamScope on_map_stream(m, pipelined);
-        LCCRF_TRY(map_prepare(m, *delta));
-        LCCRF_TRY(delta_grow_points(m, *delta));
-    }
-    if (m->n_kf <= 0 && NT > 0) return fail(LCCRF_ERR_STATE, "the map has no keyframes");
-    FrameLaunch k;
-    k.src = FrameSource::kVisible;
-    LCCRF_TRY(check_kf_ptr(kf_ptr, B, m->n_kf, &k.kf_slice_max));
-    k.ucam = m->cam_set && m->ucam;
-    if (k.ucam) memcpy(k.cam8, m->cam8, sizeof(k.cam8));
-    k.kf_bucket = (m->n_kf + 127) / 128 * 128;
-    if (!in.vis) LCCRF_TRY(slot_alloc(ctx, in, st, in.vis, (size_t)(NT ? NT : 1) * 4));
-    if (kf_ptr && !in.kf_ptr) LCCRF_TRY(slot_alloc(ctx, in, st, in.kf_ptr, (size_t)(B + 1) * 4));
-    k.vis = in.vis;
-    k.kf_ptr = kf_ptr ? in.kf_ptr : nullptr;
-    k.map = m;
-    in.has_delta = false;
-    if (delta) {
-        if (pipelined) {
-            LCCRF_TRY(delta_stage(*delta, m->kp_stride, true, (char *)in.stage, st, &in.delta));
-            in.has_delta = true;  // applied on the map's stream once the upload has landed (frames_run_slot)
-        } else {
-            DeltaDev dd;
-            LCCRF_TRY(delta_stage(*delta, m->kp_stride, false, (char *)in.stage, st, &dd));
-            LCCRF_TRY(map_apply_dev(m, dd, delta->kf_count > 0 ? delta->kf_keypoints : nullptr));
-        }
-    }
-    if (kf_ptr) LCCRF_CUDA(cudaMemcpyAsync(in.kf_ptr, kf_ptr, (size_t)(B + 1) * 4, cudaMemcpyHostToDevice, st));
-    if (NT > 0) LCCRF_CUDA(cudaMemcpyAsync(in.vis, point_id, (size_t)NT * 4, cudaMemcpyHostToDevice, st));
-    return frames_upload_finish(fr, in, st, kp2d, k);
-}
-
 static bool delta_empty(const lccrf_map_delta &d) {
     return d.kf_count == 0 && d.n_pose == 0 && d.n_xyz == 0 && d.n_erase == 0 && d.n_bad == 0 && d.n_add == 0;
 }
 
-// frame points of several resident maps into input set `in` on stream `st`: map m serves problems [map_prob[m],
-// map_prob[m+1]) and takes its delta (deltas[m], optional) first.  The unary runs over a padded point space in which
-// every non-empty segment starts at a multiple of 256 points (unary_map_points_visible_multi).
+// frame points of resident maps into input set `in` on stream `st`: map m serves problems [map_prob[m], map_prob[m+1])
+// and takes its delta (deltas[m], optional; one whose counts are all zero is skipped) first.  With several maps the
+// unary runs over a padded point space in which every non-empty segment starts at a multiple of 256 points
+// (unary_map_points_visible).
 static int frames_upload_visible_maps(lccrf_frames *fr, FrameInputs &in, cudaStream_t st, int n_maps, lccrf_map *const *maps,
                                       const lccrf_map_delta *deltas, const int *map_prob, const int *point_id,
                                       const float *kp2d, const int *kf_ptr) {
@@ -396,10 +340,10 @@ static int frames_upload_visible_maps(lccrf_frames *fr, FrameInputs &in, cudaStr
     for (int m = 0; m < n_maps; m++)
         if (map_prob[m + 1] < map_prob[m]) return fail(LCCRF_ERR_ARG, "map_prob must be non-decreasing");
     const bool pipelined = st != ctx->stream;
-    auto has_delta = [&](int m) { return deltas && !delta_empty(deltas[m]); };
+    auto with_delta = [&](int m) { return deltas && !delta_empty(deltas[m]); };
     size_t need = 0;
     for (int m = 0; m < n_maps; m++)
-        if (has_delta(m)) need += delta_stage_bytes(deltas[m], ms[m]->kp_stride, true);  // (a multiple of 256 bytes)
+        if (with_delta(m)) need += delta_stage_bytes(deltas[m], ms[m]->kp_stride, true);  // (a multiple of 256 bytes)
     if (need > in.stage_cap) {
         // rare (first steps): cudaFree waits for the device, so nothing still reads the old block
         if (in.stage) LCCRF_CUDA(cudaFree(in.stage));
@@ -410,8 +354,9 @@ static int frames_upload_visible_maps(lccrf_frames *fr, FrameInputs &in, cudaStr
         in.stage_cap = cap;
     }
     for (int m = 0; m < n_maps; m++) {
-        if (!has_delta(m)) continue;
-        // as frames_upload_visible, per map: pipelined, the bookkeeping is stream-ordered on that map's stream
+        if (!with_delta(m)) continue;
+        // host-side bookkeeping + capacity growth.  Pipelined: stream-ordered on the map's stream behind the last access
+        // of the context's stream (an array that moves is freed there, and the previous step's unary may still read it)
         LCCRF_TRY(pipelined ? map_begin_async_mut(ms[m]) : map_begin_main_access(ms[m]));
         MapStreamScope on_map_stream(ms[m], pipelined);
         LCCRF_TRY(map_prepare(ms[m], deltas[m]));
@@ -440,12 +385,25 @@ static int frames_upload_visible_maps(lccrf_frames *fr, FrameInputs &in, cudaStr
     pstart.push_back(k.np);
     k.n_seg = (int)count.size();
     k.ucam = k.n_seg > 0 && ucam;
+    if (n_maps == 1 && k.ucam) memcpy(k.cam8, ms[0]->cam8, sizeof(k.cam8));  // (kernel parameters of the one-map unary)
+    // The segment table (several maps; one map runs the single-map unary, which reads none) and the kf_ptr pairs go up
+    // from the slot's pinned buffer in one copy.  The slot is idle here -- its last submission was waited for, or its
+    // synchronous upload synchronised -- so no copy still reads the buffer.
+    const size_t tb = n_maps > 1 ? unary_seg_table_bytes(k.n_seg) : 0, pb = kf_ptr ? (size_t)2 * B * 4 : 0;
+    if (tb + pb > in.tab_cap) {  // (a new table pointer: the slot's next run sees a new launch key)
+        LCCRF_TRY(slot_alloc(ctx, in, st, in.tab, tb + pb));
+        if (in.h_tab) LCCRF_CUDA(cudaFreeHost(in.h_tab));
+        in.h_tab = nullptr;
+        in.tab_cap = 0;
+        LCCRF_CUDA(cudaHostAlloc(&in.h_tab, tb + pb, cudaHostAllocDefault));
+        in.tab_cap = tb + pb;
+    }
+    if (tb) unary_seg_table(k.n_seg, pstart.data(), cstart.data(), count.data(), hdr.data(), cams.data(), in.h_tab);
     // kf_ptr: within segment m, the slices of its problems in that map's keyframes -- they start at 0, do not decrease, and
     // the segment's last problem ends at the map's keyframe count; kf_ptr[B] = that count for the last problem's map.
     // The kernel reads a {first, end} pair per problem.
-    std::vector<int> pairs;
     if (kf_ptr) {
-        pairs.resize((size_t)2 * B);
+        int *pairs = (int *)((char *)in.h_tab + tb);
         for (int m = 0; m < n_maps; m++) {
             const int p0 = map_prob[m], p1 = map_prob[m + 1], n = ms[m]->n_kf;
             if (p1 == p0) continue;
@@ -461,25 +419,17 @@ static int frames_upload_visible_maps(lccrf_frames *fr, FrameInputs &in, cudaStr
         }
     }
     if (!in.vis) LCCRF_TRY(slot_alloc(ctx, in, st, in.vis, (size_t)(NT ? NT : 1) * 4));
-    if (kf_ptr && !in.kf_pair) LCCRF_TRY(slot_alloc(ctx, in, st, in.kf_pair, (size_t)2 * B * 4));
-    const size_t tb = unary_seg_table_bytes(k.n_seg);
-    if (tb > in.seg_tab_cap) {  // (a new table pointer: the slot's next run sees a new launch key)
-        LCCRF_TRY(slot_alloc(ctx, in, st, in.seg_tab, tb));
-        in.seg_tab_cap = tb;
-    }
-    std::vector<char> tab(tb);
-    unary_seg_table(k.n_seg, pstart.data(), cstart.data(), count.data(), hdr.data(), cams.data(), tab.data());
     k.vis = in.vis;
-    k.kf_ptr = kf_ptr ? in.kf_pair : nullptr;
+    k.kf_ptr = kf_ptr ? (const int *)((char *)in.tab + tb) : nullptr;
     k.maps = ms;
     k.map_prob.assign(map_prob, map_prob + n_maps + 1);
-    k.segs = in.seg_tab;
+    k.segs = tb ? in.tab : nullptr;
     // every delta at its own 256-byte aligned offset of the slot's stage buffer
     in.delta_maps.clear();
     in.deltas.clear();
     size_t off = 0;
     for (int m = 0; m < n_maps; m++) {
-        if (!has_delta(m)) continue;
+        if (!with_delta(m)) continue;
         char *base = (char *)in.stage + off;
         off += delta_stage_bytes(deltas[m], ms[m]->kp_stride, true);
         DeltaDev dd;
@@ -491,8 +441,7 @@ static int frames_upload_visible_maps(lccrf_frames *fr, FrameInputs &in, cudaStr
             LCCRF_TRY(map_apply_dev(ms[m], dd, deltas[m].kf_count > 0 ? deltas[m].kf_keypoints : nullptr));
         }
     }
-    LCCRF_CUDA(cudaMemcpyAsync(in.seg_tab, tab.data(), tb, cudaMemcpyHostToDevice, st));
-    if (kf_ptr && B) LCCRF_CUDA(cudaMemcpyAsync(in.kf_pair, pairs.data(), pairs.size() * 4, cudaMemcpyHostToDevice, st));
+    if (tb + pb) LCCRF_CUDA(cudaMemcpyAsync(in.tab, in.h_tab, tb + pb, cudaMemcpyHostToDevice, st));
     if (NT > 0) LCCRF_CUDA(cudaMemcpyAsync(in.vis, point_id, (size_t)NT * 4, cudaMemcpyHostToDevice, st));
     return frames_upload_finish(fr, in, st, kp2d, k);
 }
@@ -513,13 +462,13 @@ static int frames_enqueue(lccrf_frames *fr, const FrameLaunch &k) {
         LCCRF_TRY(potts_norm(ctx, b, b.lat[1]));
     }
     const float *cam8 = k.ucam ? k.cam8 : nullptr;
-    if (k.src == FrameSource::kVisible) {
-        LCCRF_TRY(unary_map_points_visible(ctx, NT, k.vis, k.map->d_hdr, k.kf_bucket, fr->observs, fr->error, fr->depth,
-                                           b.prob_ptr, k.kf_ptr, b.B, k.kf_slice_max, cam8));
-        LCCRF_TRY(map_end_main_access(k.map));  // the map may change from here on (the next step's delta, on the map's stream)
-    } else if (k.src == FrameSource::kVisibleMaps) {
-        LCCRF_TRY(unary_map_points_visible_multi(ctx, k.np, k.n_seg, k.segs, k.vis, k.kf_bucket, fr->observs, fr->error,
-                                                 fr->depth, b.prob_ptr, k.kf_ptr, b.B, k.kf_slice_max, k.ucam));
+    if (k.src == FrameSource::kVisibleMaps) {
+        // one map runs the single-map unary, which spills much less than the several-map one
+        const bool one = k.maps.size() == 1;
+        LCCRF_TRY(unary_map_points_visible(ctx, one ? NT : k.np, k.vis, one ? k.maps[0]->d_hdr : nullptr, k.n_seg, k.segs,
+                                           k.kf_bucket, fr->observs, fr->error, fr->depth, b.prob_ptr, k.kf_ptr, b.B,
+                                           k.kf_slice_max, cam8));
+        // the maps may change from here on (the next step's deltas, on the maps' streams)
         for (DevMap *m : k.maps) LCCRF_TRY(map_end_main_access(m));
     } else if (k.src != FrameSource::kDirect) {
         LCCRF_TRY(unary_pack_kf(ctx, k.kf_packed, k.kf_pose, k.kf_intr, k.kf_bounds, k.nKF));
@@ -564,18 +513,8 @@ static int frames_run_slot(lccrf_frames *fr, FrameInputs &in, cudaStream_t uploa
         // the capture pass synchronises; make sure the upload has landed first
         LCCRF_CUDA(cudaStreamSynchronize(upload_stream));
     }
-    if (in.has_delta) {
-        // this step's map changes: plain launches on the map's own stream, behind the upload and behind the previous
-        // step's unary -- they run beside that step's lattice builds and mean-field iterations
-        in.has_delta = false;
-        LCCRF_CUDA(cudaStreamWaitEvent(k.map->mstream, in.up_done, 0));
-        {
-            MapStreamScope on_map_stream(k.map);
-            LCCRF_TRY(map_apply_dev(k.map, in.delta, nullptr));
-        }
-        LCCRF_TRY(map_end_async_mut(k.map));
-    }
-    // several maps: each map's delta on that map's stream; the run waits for all of them
+    // this step's map changes: plain launches on each map's own stream, behind the upload and behind the previous step's
+    // unary -- they run beside that step's lattice builds and mean-field iterations; the run waits for all of them
     for (size_t i = 0; i < in.deltas.size(); i++) {
         DevMap *m = in.delta_maps[i];
         LCCRF_CUDA(cudaStreamWaitEvent(m->mstream, in.up_done, 0));
@@ -587,9 +526,7 @@ static int frames_run_slot(lccrf_frames *fr, FrameInputs &in, cudaStream_t uploa
     }
     in.deltas.clear();
     in.delta_maps.clear();
-    if (k.src == FrameSource::kVisible) LCCRF_TRY(map_begin_main_access(k.map));
-    if (k.src == FrameSource::kVisibleMaps)
-        for (DevMap *m : k.maps) LCCRF_TRY(map_begin_main_access(m));
+    for (DevMap *m : k.maps) LCCRF_TRY(map_begin_main_access(m));
     LCCRF_TRY(graph_run(ctx, in.graph, [&] { return frames_enqueue(fr, k); }));
     fr->ran = true;
     return LCCRF_OK;
@@ -695,8 +632,8 @@ static void frame_inputs_release(Ctx *ctx, FrameInputs &in) {
     dev_free(ctx, in.kf_packed);
     dev_free(ctx, in.kf_ptr);
     dev_free(ctx, in.vis);
-    dev_free(ctx, in.seg_tab);
-    dev_free(ctx, in.kf_pair);
+    dev_free(ctx, in.tab);
+    if (in.h_tab) cudaFreeHost(in.h_tab);
     dev_free(ctx, in.out_stage);
     if (in.res_ready) cudaEventDestroy(in.res_ready);
     dev_free(ctx, in.p4);
@@ -800,12 +737,8 @@ int lccrf_frames_set_map_inputs_indexed(lccrf_frames *fr, const float *xyz, cons
 int lccrf_frames_set_visible(lccrf_frames *fr, lccrf_map *map, const lccrf_map_delta *delta, const int *point_id,
                              const float *kp2d, const int *kf_ptr) {
     if (!fr) return fail(LCCRF_ERR_ARG, "frames is NULL");
-    LCCRF_CUDA(cudaSetDevice(fr->ctx->device));
-    LCCRF_TRY(frames_check_idle(fr));
-    LCCRF_TRY(frames_upload_visible(fr, fr->in[0], fr->ctx->stream, map, delta, point_id, kp2d, kf_ptr));
-    // the host arrays (delta included) are free on return
-    LCCRF_CUDA(cudaStreamSynchronize(fr->ctx->stream));
-    return LCCRF_OK;
+    const int map_prob[2] = {0, fr->b.B};
+    return lccrf_frames_set_visible_maps(fr, 1, &map, delta, map_prob, point_id, kp2d, kf_ptr);
 }
 
 int lccrf_frames_set_visible_maps(lccrf_frames *fr, int n_maps, lccrf_map *const *maps, const lccrf_map_delta *deltas,
@@ -913,15 +846,9 @@ int lccrf_frames_submit_map_indexed(lccrf_frames *fr, int slot, const float *xyz
 
 int lccrf_frames_submit_visible(lccrf_frames *fr, int slot, lccrf_map *map, const lccrf_map_delta *delta, const int *point_id,
                                 const float *kp2d, const int *kf_ptr, short *map_out, float *prob_out) {
-    FrameInputs *in = nullptr;
-    PhaseTimer tm(fr && fr->ctx->opt_trace);
-    LCCRF_TRY(frames_submit_prologue(fr, slot, &in));
-    tm.mark("prologue");
-    LCCRF_TRY(frames_upload_visible(fr, *in, fr->ctx->copy_stream, map, delta, point_id, kp2d, kf_ptr));
-    tm.mark("upload");
-    const int rc = frames_submit_epilogue(fr, slot, *in, map_out, prob_out);
-    tm.mark("apply+run+results");
-    return rc;
+    if (!fr) return fail(LCCRF_ERR_ARG, "frames is NULL");
+    const int map_prob[2] = {0, fr->b.B};
+    return lccrf_frames_submit_visible_maps(fr, slot, 1, &map, delta, map_prob, point_id, kp2d, kf_ptr, map_out, prob_out);
 }
 
 int lccrf_frames_submit_visible_maps(lccrf_frames *fr, int slot, int n_maps, lccrf_map *const *maps,
@@ -1055,10 +982,9 @@ int lccrf_frames_algorithmic_bytes(lccrf_frames *fr, double *total, double *per_
     const FrameLaunch &k = fr->in[fr->last_slot].launch;
     long long nnz = k.nnz;
     int nKF = k.nKF;
-    if (k.src == FrameSource::kVisible || k.src == FrameSource::kVisibleMaps) {  // observations of the visible points: counted on the device
+    if (k.src == FrameSource::kVisibleMaps) {  // observations of the visible points: counted on the device
         // (map, first point, end point) of every segment
         std::vector<std::pair<DevMap *, std::pair<int, int>>> seg;
-        if (k.src == FrameSource::kVisible) seg.push_back({k.map, {0, fr->b.NT}});
         for (size_t m = 0; m < k.maps.size(); m++)
             seg.push_back({k.maps[m], {fr->b.h_prob_ptr[k.map_prob[m]], fr->b.h_prob_ptr[k.map_prob[m + 1]]}});
         nKF = 0;
